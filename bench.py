@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--config 2|3|4|5]   # this repo's CUDA engine
     python bench.py --impl reference --gpus N --steps K ...             # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                              # also write the last timed step's outputs
 
 One "step" = one pass of the hot path over one batch of synthetic input.  `--config` selects the BASELINE.json
 configuration (1-based, as SURVEY.md section 8d numbers them; default 3, the one the samples/sec metric is quoted on):
@@ -263,6 +264,26 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ engine arm
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(d: str, arrays: dict):
+    """Write each array as `d/<name>.npy` (float32 or float64), at most DUMP_BYTES in all.  When the arrays do not fit, each
+    one of more than 2^20 elements is replaced by a fixed seeded sample of its flattened elements, with the sampled flat
+    positions in `d/<name>_index.npy`.  The inputs are seeded, so two builds can be compared file for file."""
+    os.makedirs(d, exist_ok=True)
+    big = {k for k, a in arrays.items() if a.size > 1 << 20}
+    small_bytes = sum(a.nbytes for k, a in arrays.items() if k not in big) + 2048 * len(arrays)     # (.npy headers)
+    big_bytes = sum(arrays[k].nbytes for k in big)
+    for name, a in arrays.items():
+        if name in big and small_bytes + big_bytes > DUMP_BYTES:
+            k = int(a.size * (DUMP_BYTES - small_bytes) / big_bytes / (1 + 8 / a.itemsize))   # values + float64 positions
+            idx = np.sort(np.random.default_rng(0).choice(a.size, k, replace=False))
+            np.save(os.path.join(d, name + "_index.npy"), idx.astype(np.float64))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 class Dist:
     def __init__(self, torch):
         self.rank, self.world, self.local = dist_env()
@@ -469,7 +490,11 @@ def run_engine(args):
     # The reference-facing call returns what piper::synthesize returns: peak-normalised int16 samples (piper.cpp:411-431),
     # here produced on the GPU (pb200_synthesize_int16), so 2 bytes per sample cross PCIe.  The fp32 variant of the same
     # call (pb200_synthesize_batch, 4 bytes per sample) is timed beside it.
-    def e2e_leg(call, bytes_per_sample):
+    # Both legs run the staged leg's inputs (same ids, scales and noise seed); what the last timed step of each returned
+    # to its caller - the concatenated waveforms and the per-utterance sample counts - is what --dump-outputs writes.
+    outputs = {}
+
+    def e2e_leg(call, bytes_per_sample, name):
         for _ in range(3):
             call()
         D.barrier()
@@ -480,9 +505,16 @@ def run_engine(args):
             n += int(counts.sum())
         D.barrier()
         secs = D.max(time.perf_counter() - t0)
+        if args.dump_outputs:
+            outputs[name] = flat.astype(np.float32)        # a copy: the library reuses its host buffer on the next call
+            outputs["samples_per_utterance"] = counts.astype(np.float64)
         return D.sum(float(n)) / secs, secs, n // steps * bytes_per_sample
-    e2e_value, e2e_s, d2h_audio = e2e_leg(lambda: voice.synthesize_int16(ids_list, SCALES, seed=4242, copy=False), 2)
-    e2e_f32, e2e_f32_s, d2h_f32 = e2e_leg(lambda: voice.synthesize_batch(ids_list, SCALES, seed=4242, copy=False), 4)
+    e2e_value, e2e_s, d2h_audio = e2e_leg(lambda: voice.synthesize_int16(ids_list, SCALES, seed=4242, copy=False), 2,
+                                          "audio_int16")
+    e2e_f32, e2e_f32_s, d2h_f32 = e2e_leg(lambda: voice.synthesize_batch(ids_list, SCALES, seed=4242, copy=False), 4,
+                                          "audio")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
     tp = (259 + 3) // 4 * 4
     h2d = B * tp * 4 + B * 4 + B * 8 + 24       # ids (int32, padded pitch) + lengths + output offsets + call parameters
     d2h = d2h_audio + B * 4                     # int16 audio + the per-item output lengths
@@ -567,13 +599,15 @@ def run_generator_sweep(args, D, torch):
         dev_ms, t0 = 0.0, time.perf_counter()
         launches0 = engine.launch_count()
         for _ in range(args.steps):
-            voice.vocode(z)
+            audio, _ = voice.vocode(z)
             dev_ms += voice.stage_times()[4]
         D.barrier()
         wall = D.max(time.perf_counter() - t0)
         launches = (engine.launch_count() - launches0) / args.steps
         if rank == 0 and top:
             clocks = sampler.stop()
+            if args.dump_outputs:                        # the headline batch's waveforms [B, 65536] of the last step
+                dump_outputs(args.dump_outputs, {"audio": audio})
         ms = D.max(dev_ms) / args.steps
         n = B * 256 * voice.hop
         gbs = (act * B + wb) / (ms * 1e-3) / 1e9
@@ -630,6 +664,8 @@ def main():
     ap.add_argument("--arch", default="medium", choices=["medium", "high"], help="decoder of the generator sweep (config 5)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="developer A/B runs: no pipe-peak measurement, streaming leg or CPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last step to DIR/<name>.npy "
+                    "(float32 / float64, at most 64 MB; seeded inputs, so runs of two builds compare output for output)")
     ap.add_argument("--cpu-worker", type=int, default=0)
     ap.add_argument("--cpu-utts", type=int, default=2)
     ap.add_argument("--cpu-threads", type=int, default=8)

@@ -1,6 +1,7 @@
 """Mint the golden fixtures under tests/golden/ from the REFERENCE's own PyTorch model source.
 
 Run in the build container only (needs /root/reference):  python -m oracle.make_golden
+(`python -m oracle.make_golden reference-checks` mints tests/golden/reference/ only.)
 Each fixture stores the inputs (phoneme ids, scales, injected noise) and the outputs of
 `SynthesizerTrn.infer` (/root/reference/src/python/piper_train/vits/models.py:681-722) run on
 CPU fp32 through oracle/ref_bridge.py: per-id frame counts, the latent z and the waveform.
@@ -108,5 +109,67 @@ def mint_streaming():
     print("stream_tiny:", r["y_len"], "frames ->", [len(p) for p in pieces])
 
 
+# The cases tests/test_oracle.py compares with the reference source (voice tag, phonemes, scales); their outputs are stored
+# under tests/golden/reference/ so that the comparison runs without the reference tree.
+SOURCE_CASES = [("real:test_voice", 0, (0.667, 1.0, 0.8)), ("synthetic:tiny:1234", 40, (0.667, 1.3, 0.8)),
+                ("synthetic:tiny-high:1234", 12, (0.3, 0.8, 1.0)), ("synthetic:tiny-ms:1234", 25, (0.667, 1.0, 0.8))]
+REF_OUT = os.path.join(OUT, "reference")
+SAMPLES = 1024
+
+
+def sample(out, key, a, seed):
+    """Store the shape of `a` and a fixed seeded sample of its elements (flat indices and values) under `key`."""
+    a = np.asarray(a, np.float32)
+    idx = np.sort(np.random.default_rng(seed).choice(a.size, min(a.size, SAMPLES), replace=False)).astype(np.int32)
+    out.update({f"{key}.shape": np.asarray(a.shape, np.int64), f"{key}.idx": idx, f"{key}.val": a.reshape(-1)[idx]})
+
+
+def mint_reference_checks():
+    """Outputs of the reference's own model source and streaming chunk loop for the inputs the tests draw, plus the
+    test voice's config and its pre-phonemized en-us sentences (small text fixtures)."""
+    import shutil
+    from oracle.vits_oracle import Oracle
+    assert ref_bridge.available(), "needs the reference source tree"
+    os.makedirs(REF_OUT, exist_ok=True)
+    shutil.copyfile(REAL + ".json", os.path.join(REF_OUT, "test_voice.onnx.json"))
+    shutil.copyfile(FIXTURES, os.path.join(REF_OUT, "test_en-us.jsonl"))
+    lines = [json.loads(l) for l in open(FIXTURES)]
+    out = {}
+    for i, (tag, n_ph, scales) in enumerate(SOURCE_CASES):
+        path = REAL if tag.startswith("real:") else voicegen.cached_voice(tag.split(":")[1], int(tag.split(":")[2]))
+        spec, w, _ = load_voice(path)
+        net = ref_bridge.build_reference_model(spec, w)
+        ids = lines[3]["phoneme_ids"] if tag.startswith("real:") else voicegen.benchmark_ids(n_ph, seed=17)
+        rng = np.random.default_rng(11)
+        eps_dp = rng.standard_normal((2, len(ids))).astype(np.float32)
+        eps_z = rng.standard_normal((spec.inter, 6 * len(ids))).astype(np.float32)
+        sid = 2 if spec.n_speakers > 1 else None
+        r = ref_bridge.reference_infer(net, ids, scales, eps_dp, eps_z, sid=sid)
+        out[f"{tag}.ids"] = np.asarray(ids, np.int64)
+        out[f"{tag}.w_ceil"] = r["w_ceil"].astype(np.int32)
+        out[f"{tag}.weights_sha256"] = np.array(weights_digest(w))
+        for j, k in enumerate(("z_p", "z", "o")):
+            sample(out, f"{tag}.{k}", r[k], 100 * i + j)
+        print(f"{tag}: ids={len(ids)} frames={r['y_len']}")
+    np.savez_compressed(os.path.join(REF_OUT, "source_cases.npz"), **out)
+
+    # SpeechStreamer.chunk of the reference on the oracle's latent (tests/test_oracle.py draws the same input)
+    path = voicegen.cached_voice("tiny")
+    spec, w, attrs = load_voice(path)
+    orc = Oracle(spec, w, attrs)
+    net = ref_bridge.build_reference_model(spec, w)
+    z_p = orc.encode(voicegen.benchmark_ids(70, seed=5), (0.667, 1.0, 0.8))
+    pieces = ref_bridge.reference_stream_chunks(net, z_p, z_p.shape[1], 45, 10)
+    out = dict(piece_lens=np.asarray([len(p) for p in pieces], np.int64), weights_sha256=np.array(weights_digest(w)))
+    sample(out, "z_p", z_p, 1000)
+    sample(out, "audio", np.concatenate(pieces), 1001)
+    np.savez_compressed(os.path.join(REF_OUT, "stream_chunk_loop.npz"), **out)
+    print("stream_chunk_loop:", [len(p) for p in pieces])
+
+
 if __name__ == "__main__":
-    main()
+    import sys
+    if sys.argv[1:] == ["reference-checks"]:
+        mint_reference_checks()
+    else:
+        main()

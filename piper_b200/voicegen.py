@@ -26,6 +26,7 @@ from __future__ import annotations
 import json
 import math
 import os
+import tempfile
 from typing import Dict, List, Tuple
 
 import numpy as np
@@ -240,7 +241,9 @@ def write_voice(path: str, arch: str = "medium", seed: int = 1234, n_vocab: int 
 
 
 def cached_voice(arch: str = "medium", seed: int = 1234, root: str | None = None) -> str:
-    root = root or os.environ.get("PIPER_B200_VOICE_CACHE", "/tmp/piper_b200_voices")
+    # per user: the machine's temporary directory may be shared, and another user's cache is not writable
+    root = root or os.environ.get("PIPER_B200_VOICE_CACHE",
+                                  os.path.join(tempfile.gettempdir(), f"piper_b200_voices-{os.getuid()}"))
     path = os.path.join(root, f"synthetic-{arch}-s{seed}.onnx")
     if not (os.path.exists(path) and os.path.exists(path + ".json")):
         write_voice(path, arch, seed)

@@ -8,32 +8,22 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REF_ROOT = "/root/reference"
-REAL_VOICE_CANDIDATES = [
-    os.path.join(REF_ROOT, "etc", "test_voice.onnx"),
-    os.path.join(ROOT, "oracle", "_ref", "voice", "test_voice.onnx"),
-]
+# the reference's test voice (27 MB, too large to store) where build() staged it; its config and sentences are stored
+REAL_VOICE = os.path.join(ROOT, "oracle", "_ref", "voice", "test_voice.onnx")
+REAL_VOICE_CONFIG = os.path.join(GOLDEN, "reference", "test_voice.onnx.json")
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a B200 (run with -m gpu on the GPU box)")
-    config.addinivalue_line("markers", "needs_reference: imports the reference source from /root/reference")
 
 
 def real_voice_path():
-    for p in REAL_VOICE_CANDIDATES:
-        if os.path.exists(p):
-            return p
-    return None
+    return REAL_VOICE if os.path.exists(REAL_VOICE) else None
 
 
 def real_fixture_lines():
     import json
-    for p in (os.path.join(REF_ROOT, "etc", "test_sentences", "test_en-us.jsonl"),
-              os.path.join(ROOT, "oracle", "_ref", "voice", "test_en-us.jsonl")):
-        if os.path.exists(p):
-            return [json.loads(l) for l in open(p)]
-    return None
+    return [json.loads(l) for l in open(os.path.join(GOLDEN, "reference", "test_en-us.jsonl"))]
 
 
 @pytest.fixture(scope="session")

@@ -293,7 +293,7 @@ def test_streaming_encode_decode_split():
     assert len(pcm) == len(out) and all(len(b) == 2 * len(p) for b, p in zip(pcm, out))
 
 
-def test_cpp_shim_test_program():
+def test_cpp_shim_test_program(tmp_path):
     """The reference's only automated test (src/cpp/test.cpp) restated against the piper.hpp-compatible shim."""
     import subprocess
     from conftest import ROOT
@@ -301,10 +301,8 @@ def test_cpp_shim_test_program():
     voice = real_voice_path()
     if voice is None or not os.path.exists(exe):
         pytest.skip("shim test program or reference voice not staged")
-    sentences = os.path.join(os.path.dirname(voice), "test_en-us.jsonl")
-    if not os.path.exists(sentences):
-        sentences = "/root/reference/etc/test_sentences/test_en-us.jsonl"
-    out = os.path.join("/tmp", "piper_b200_shim_test.wav")
+    sentences = os.path.join(GOLDEN, "reference", "test_en-us.jsonl")
+    out = str(tmp_path / "shim_test.wav")
     r = subprocess.run([exe, voice, sentences, out, "1"], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0, r.stderr
     assert "OK" in r.stdout and os.path.getsize(out) >= 10000

@@ -77,7 +77,7 @@ def test_fused_mrf_ragged_batch():
 
 
 _CHILD = r"""
-import json, os, sys
+import json, os, sys, tempfile
 import numpy as np
 sys.path.insert(0, {root!r})
 from oracle.voice_loader import load_voice
@@ -95,7 +95,8 @@ for arch, n_ph, batch in (("tiny", 20, 1), ("medium", 64, 1), ("medium", 128, 32
     wavs, _ = v.synthesize_batch(ids, (0.667, 1.0, 0.8), eps_dp=eps_dp, eps_z=np.stack(eps_z))
     worst = 0.0
     for b in sorted(set([0, batch - 1])):
-        cache = f"/tmp/piper_b200_exp_ref_{{arch}}_{{n_ph}}_{{batch}}_{{b}}.npy"     # the oracle's answer is the same for every variant
+        # the oracle's answer is the same for every variant (cached per user: the temporary directory may be shared)
+        cache = os.path.join(tempfile.gettempdir(), f"piper_b200_exp_ref-{{os.getuid()}}_{{arch}}_{{n_ph}}_{{batch}}_{{b}}.npy")
         if os.path.exists(cache):
             ref = np.load(cache)
         else:

@@ -9,7 +9,7 @@ import struct
 import numpy as np
 import pytest
 
-from conftest import ROOT, real_fixture_lines, real_voice_path
+from conftest import REAL_VOICE_CONFIG, ROOT, real_fixture_lines, real_voice_path
 from piper_b200 import host, onnx_wire, voicegen
 
 
@@ -179,10 +179,7 @@ def test_no_cpu_fallback(lib_built):
 # ------------------------------------------------------------------ host logic
 def test_phonemes_to_ids_reproduces_reference_fixtures():
     lines = real_fixture_lines()
-    path = real_voice_path()
-    if lines is None or path is None:
-        pytest.skip("reference fixtures not staged")
-    cfg = host.VoiceConfig.load(path + ".json")
+    cfg = host.VoiceConfig.load(REAL_VOICE_CONFIG)
     assert cfg.sample_rate == 16000 and cfg.num_speakers == 1
     for l in lines:
         assert host.phonemes_to_ids(l["phonemes"], cfg.phoneme_id_map) == l["phoneme_ids"]
