@@ -65,12 +65,12 @@ typedef struct pb200_noise {
 /* Parse `onnx_path`, pack the weights and upload them to CUDA device `device`. */
 int pb200_voice_load(const char* onnx_path, int device, pb200_voice** out);
 /* Multi-GPU load (SURVEY §8e): every rank parses the file (host only), rank 0 uploads, the other ranks pass
- * PB200_LOAD_NO_UPLOAD and receive the two packed blobs (fp32 layout, split-precision tensor-core layout) by an
- * NCCL broadcast over NVLink into the device buffers returned by pb200_voice_weight_buffers.  The hot path itself
- * has no collective: utterances are independent. */
+ * PB200_LOAD_NO_UPLOAD and receive the packed fp32 weight blob by an NCCL broadcast over NVLink into the device
+ * buffer returned by pb200_voice_weight_buffers.  Every rank packs its own tensor-core weights from its host parse on
+ * first use.  The hot path itself has no collective: utterances are independent. */
 #define PB200_LOAD_NO_UPLOAD 1
 int pb200_voice_load_ex(const char* onnx_path, int device, int32_t flags, pb200_voice** out);
-int pb200_voice_weight_buffers(pb200_voice* v, void** fp32, int64_t* fp32_bytes, void** mma, int64_t* mma_bytes);
+int pb200_voice_weight_buffers(pb200_voice* v, void** fp32, int64_t* fp32_bytes);
 void pb200_voice_free(pb200_voice* v);
 int pb200_voice_get_info(const pb200_voice* v, pb200_voice_info* info);
 
@@ -128,35 +128,27 @@ int pb200_profile_read(pb200_voice* v, char* buf, int64_t cap);
  * (tag, tensor-core flag, microseconds, layer shape, algorithmic bytes / FLOP).  Fails if cap is too small. */
 int pb200_profile_read_launches(pb200_voice* v, char* buf, int64_t cap);
 
-/* Select which layer families run on the tcgen05 tensor cores (split precision): bit 0 = generator (bf16x3),
- * bit 1 = flow (tf32x3), bit 2 = text encoder (tf32x3), bit 3 = duration predictor (tf32x3); cleared bits use the fp32
- * CUDA-core kernel.  Default 15.  The tensor core truncates (RZ) when adding into its fp32 accumulator; the tf32x3 layers therefore split
- * K into 3 chains plus a separate accumulator for the correction terms and combine them in fp32 RN in the epilogue,
- * which restores fp32-grade accuracy on the ill-conditioned real test voice (DESIGN.md §Precision).
- * Env PIPER_B200_MMA=<mask> sets the default at load. */
+/* Select which layer families run on the tcgen05 tensor cores (split precision, fp16x3 by default): bit 0 = generator,
+ * bit 1 = flow, bit 2 = text encoder, bit 3 = duration predictor, bit 4 = the generator's MRF stages fused into one
+ * launch each; cleared bits use the fp32 CUDA-core kernel.  Default 31.  The tensor core truncates (RZ) when adding into
+ * its fp32 accumulator; the long reductions of the flow, encoder and duration predictor therefore run in 2 K-chains,
+ * each with its own correction accumulator, combined in fp32 RN in the epilogue, which keeps fp32-grade accuracy on the
+ * ill-conditioned real test voice (DESIGN.md §3).  Env PIPER_B200_MMA=<mask> sets the default at load. */
 int pb200_set_mma(pb200_voice* v, int32_t mask);
-/* Kernel-level test hook: one Conv1d (same-padded, pad = dil*(k-1)/2) on host arrays through the chosen
- * back end (0 = CUDA-core kernel, 1 = tensor cores bf16x3, 2 = tensor cores tf32x3).  x [B][ci][L], w [co][ci][k], bias [co] or NULL,
- * pre_slope != 0 applies leaky-relu to the input, resid [B][co][L] or NULL is added, y [B][co][L]. */
+/* Kernel-level test hook: one Conv1d (same-padded, pad = dil*(k-1)/2) on host arrays through the chosen back end:
+ * 0 = CUDA-core kernel; tensor cores 1 (or 3) = bf16x3, 2 (or 4) = tf32x3 with 2 K-chains, 5 = fp16x3 with 1 chain,
+ * 6 = fp16x3 with 2 chains.  Any other value is an error.  x [B][ci][L], w [co][ci][k], bias [co] or NULL, pre_slope != 0 applies
+ * leaky-relu to the input, resid [B][co][L] or NULL is added, y [B][co][L]. */
 int pb200_debug_conv1d(int32_t backend, const float* x, int32_t B, int32_t ci, int32_t L, const float* w,
                        const float* bias, int32_t co, int32_t k, int32_t dil, float pre_slope, const float* resid,
                        float* y);
 
-/* Host-only (no GPU): tiling and packed weights of the EXPERIMENTAL fused MRF stage (csrc/mrf_fused.cu, engine mask bit
- * 16, off by default) for upsample stage `stage` of a voice; fuse_post != 0 plans it with conv_post + tanh fused behind it.
+/* Host-only (no GPU): tiling and packed weights of the fused MRF stage (csrc/mrf_fused.cu, engine mask bit 16) for
+ * upsample stage `stage` of a voice; fuse_post != 0 plans it with conv_post + tanh fused behind it.
  * plan = {ok, n_chains, n_steps, pair, hv, to, k[3], dil[3][6], post_k}; w = bf16 tap tiles in consumption order,
  * bias = [step][chain][32].  w / bias may be NULL to query sizes. */
 int pb200_debug_mrf_pack(const char* onnx_path, int32_t stage, int32_t fuse_post, int32_t plan[32], uint8_t* w,
                          int64_t* w_bytes, float* bias, int64_t* n_bias);
-
-/* Host-only: the tensor-core tiling chosen for a layer shape.  out = {supported, rows per tile (MT), channel chunk,
- * staged rows, output rows per tile, number of row tiles, TMEM columns per accumulator, TMEM columns allocated,
- * activation slots, weight slots, accumulators per row half, dynamic shared memory bytes}. */
-int pb200_debug_mma_plan(int32_t ci, int32_t rows, int32_t k, int32_t dil, int32_t tf32, int32_t out[12]);
-
-/* Developer microbenchmark: issue `iters` tcgen05.mma (M=128, given N, bf16 or tf32, no-swizzle K-major smem operands)
- * rotating over n_acc accumulators; cycles[0] = issue time, cycles[1] = until the last one retired. */
-int pb200_debug_mma_bench(int32_t N, int32_t tf32, int32_t n_acc, int32_t iters, int32_t shift, uint64_t* cycles);
 
 void pb200_release(pb200_voice* v, const void* audio);
 

@@ -30,7 +30,7 @@ _p = C.POINTER
 SYMBOLS = {
     "pb200_voice_load": (C.c_int, [C.c_char_p, C.c_int, _p(C.c_void_p)]),
     "pb200_voice_load_ex": (C.c_int, [C.c_char_p, C.c_int, C.c_int32, _p(C.c_void_p)]),
-    "pb200_voice_weight_buffers": (C.c_int, [C.c_void_p, _p(C.c_void_p), _p(C.c_int64), _p(C.c_void_p), _p(C.c_int64)]),
+    "pb200_voice_weight_buffers": (C.c_int, [C.c_void_p, _p(C.c_void_p), _p(C.c_int64)]),
     "pb200_voice_free": (None, [C.c_void_p]),
     "pb200_voice_get_info": (C.c_int, [C.c_void_p, _p(VoiceInfo)]),
     "pb200_voice_describe": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int64]),
@@ -58,8 +58,6 @@ SYMBOLS = {
                                      _p(C.c_float)]),
     "pb200_debug_mrf_pack": (C.c_int, [C.c_char_p, C.c_int32, C.c_int32, _p(C.c_int32), _p(C.c_uint8), _p(C.c_int64), _p(C.c_float),
                                        _p(C.c_int64)]),
-    "pb200_debug_mma_plan": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _p(C.c_int32)]),
-    "pb200_debug_mma_bench": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _p(C.c_uint64)]),
     "pb200_release": (None, [C.c_void_p, C.c_void_p]),
     "pb200_set_speakers": (C.c_int, [C.c_void_p, _p(C.c_int64), C.c_int32]),
     "pb200_set_debug": (C.c_int, [C.c_void_p, C.c_int32]),

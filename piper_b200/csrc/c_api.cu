@@ -60,10 +60,10 @@ int pb200_voice_load_ex(const char* onnx_path, int device, int32_t flags, pb200_
   });
 }
 
-int pb200_voice_weight_buffers(pb200_voice* v, void** fp32, int64_t* fp32_bytes, void** mma, int64_t* mma_bytes) {
+int pb200_voice_weight_buffers(pb200_voice* v, void** fp32, int64_t* fp32_bytes) {
   return guarded([&] {
-    if (!v || !fp32 || !fp32_bytes || !mma || !mma_bytes) throw std::runtime_error("pb200_voice_weight_buffers: null argument");
-    v->engine.weight_buffers(fp32, fp32_bytes, mma, mma_bytes);
+    if (!v || !fp32 || !fp32_bytes) throw std::runtime_error("pb200_voice_weight_buffers: null argument");
+    v->engine.weight_buffers(fp32, fp32_bytes);
   });
 }
 
@@ -259,6 +259,8 @@ int pb200_debug_conv1d(int32_t backend, const float* x, int32_t B, int32_t ci, i
   return guarded([&] {
     using namespace pb200;
     if (!x || !w || !y || B <= 0 || L <= 0) throw std::runtime_error("pb200_debug_conv1d: bad argument");
+    if (backend < 0 || backend > 6)
+      throw std::runtime_error("pb200_debug_conv1d: backend " + std::to_string(backend) + " is not 0..6");
     const int Lp = (L + 3) & ~3, pad = dil * (k - 1) / 2, rows_p = (co + 3) & ~3;
     float *dx = nullptr, *dy = nullptr, *dr = nullptr, *dw = nullptr, *db = nullptr;
     int* dlen = nullptr;
@@ -292,12 +294,13 @@ int pb200_debug_conv1d(int32_t backend, const float* x, int32_t B, int32_t ci, i
       a.pre = pre_slope != 0.f ? PRE_LRELU : PRE_NONE; a.slope = pre_slope;
       a.epi = resid ? EPI_RES : EPI_BIAS;
       launch_conv1d(a, B, L, nullptr);
-    } else if (backend >= 3) {
-      // second-generation kernel (conv_mma2.cu): 3 = bf16x3, 4 = tf32x3 (2 chains), 5 = fp16x3 (1 chain), 6 = fp16x3 (2 chains)
-      const int prec = backend == 3 ? 0 : backend == 4 ? 1 : 2;
+    } else {
+      // tensor-core kernel (conv_mma2.cu): 1, 3 = bf16x3; 2, 4 = tf32x3 (2 chains); 5 = fp16x3 (1 chain); 6 = fp16x3 (2 chains)
+      const int prec = (backend == 1 || backend == 3) ? 0 : (backend == 2 || backend == 4) ? 1 : 2;
+      const int chains = (backend == 2 || backend == 4 || backend == 6) ? 2 : 1;
       Conv2Layer l;
-      if (!conv2_plan(ci, co, k, dil, prec, (backend == 4 || backend == 6) ? 2 : 1, l))
-        throw std::runtime_error("shape not supported by the second-generation tensor-core conv");
+      if (!conv2_plan(ci, co, k, dil, prec, chains, l))
+        throw std::runtime_error("shape not supported by the tensor-core conv");
       std::vector<float> pk(size_t(ci) * k * rows_p, 0.f);
       for (int i = 0; i < ci; ++i)
         for (int j = 0; j < k; ++j)
@@ -311,48 +314,11 @@ int pb200_debug_conv1d(int32_t backend, const float* x, int32_t B, int32_t ci, i
       a.ci = ci; a.rows = co; a.k = k; a.dil = dil; a.pad = pad;
       a.pre = pre_slope != 0.f ? PRE_LRELU : PRE_NONE; a.slope = pre_slope;
       a.epi = resid ? EPI_RES : EPI_BIAS;
-      if (!launch_conv2(a, l, B, L, nullptr)) throw std::runtime_error("launch too small for conv2 (set PIPER_B200_V2=2)");
-    } else {
-      MmaPlan plan;
-      if (!mma_plan(ci, co, k, dil, backend == 2, plan)) throw std::runtime_error("shape not supported by the tensor-core conv");
-      std::vector<float> pk(size_t(ci) * k * rows_p, 0.f);
-      for (int i = 0; i < ci; ++i)
-        for (int j = 0; j < k; ++j)
-          for (int o = 0; o < co; ++o) pk[(size_t(i) * k + j) * rows_p + o] = w[(size_t(o) * ci + i) * k + j];
-      std::vector<uint8_t> pm;
-      pack_conv_mma(pk.data(), ci, k, co, rows_p, plan, pm);
-      CK(cudaMalloc(&dw16, pm.size()));
-      CK(cudaMemcpy(dw16, pm.data(), pm.size(), cudaMemcpyHostToDevice));
-      MmaConvArgs m;
-      m.x = vx; m.y = vy; m.r = vr; m.w = dw16; m.bias = db; m.len = dlen; m.len_scale = 1;
-      m.ci = ci; m.rows = co; m.k = k; m.dil = dil; m.pad = pad;
-      m.pre = pre_slope != 0.f ? PRE_LRELU : PRE_NONE; m.slope = pre_slope;
-      m.epi = resid ? EPI_RES : EPI_BIAS;
-      launch_conv_mma(m, plan, B, L, nullptr);
+      launch_conv2(a, l, B, L, nullptr);
     }
     CK(cudaDeviceSynchronize());
     CK(cudaMemcpy2D(y, size_t(L) * 4, dy, size_t(Lp) * 4, size_t(L) * 4, size_t(B) * co, cudaMemcpyDeviceToHost));
     cudaFree(dx); cudaFree(dy); cudaFree(dr); cudaFree(dw); cudaFree(db); cudaFree(dlen); cudaFree(dw16);
-  });
-}
-
-int pb200_debug_mma_plan(int32_t ci, int32_t rows, int32_t k, int32_t dil, int32_t tf32, int32_t out[12]) {
-  return guarded([&] {
-    if (!out) throw std::runtime_error("pb200_debug_mma_plan: null argument");
-    pb200::MmaPlan p;
-    const bool ok = pb200::mma_plan(ci, rows, k, dil, tf32 != 0, p);
-    const int32_t v[12] = {ok, p.mt, p.kc, p.stage_rows, p.n_tile, p.n_tiles, p.acc_cols, p.tmem_cols, p.a_slots, p.w_slots,
-                           p.chains + (p.sep_corr ? 1 : 0), int32_t(p.smem)};
-    for (int i = 0; i < 12; ++i) out[i] = v[i];
-  });
-}
-
-int pb200_debug_mma_bench(int32_t N, int32_t tf32, int32_t n_acc, int32_t iters, int32_t shift, uint64_t* cycles) {
-  return guarded([&] {
-    unsigned long long o[2] = {0, 0};
-    pb200::run_mma_bench(N, tf32, n_acc, iters, shift, o);
-    cycles[0] = o[0];
-    cycles[1] = o[1];
   });
 }
 

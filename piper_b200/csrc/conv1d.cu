@@ -12,7 +12,7 @@
 // convolutions costs zero extra HBM traffic.
 //
 // fp32 FFMA keeps the 1e-3 waveform parity bar (single-pass TF32/BF16 tensor-core math does not:
-// SURVEY.md finding 7); the split-precision tcgen05 path for the large layers lives in conv_mma.cu.
+// SURVEY.md finding 7); the split-precision tcgen05 path for the large layers lives in conv_mma2.cu.
 //
 // Reference ops covered: every Conv / ConvTranspose node of the exported graph except the depthwise
 // ones (SURVEY.md App. B.1; modules.py:184-209,301-314,355-364; models.py:348-368; attentions.py:386-407).

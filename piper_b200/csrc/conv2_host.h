@@ -1,4 +1,4 @@
-// Host side of the experimental second-generation tensor-core convolution (conv2_body.inl): tiling plan, stacked weight
+// Host side of the persistent tensor-core convolution (conv2_body.inl): tiling plan, stacked weight
 // packing and launch-argument fill.  Plain C++ (no CUDA calls): shared by conv_mma2.cu and the CPU model in tests/sim.
 #pragma once
 #include <algorithm>
@@ -172,7 +172,7 @@ inline void pack(const float* wsrc, int ci, int k, int rows_p, const Plan& p, ui
 constexpr size_t kAstatSmem = size_t(212) << 10;
 inline int fill_args(MmaConvArgs& a, const Plan& p, int B, int max_len, bool tm = false, TmapDesc* td = nullptr, bool astat_ok = false,
                      size_t* smem_out = nullptr) {
-  a.n_tile = p.n_tile; a.acc_cols = p.n_tile; a.chains = p.chains; a.mh_stride = p.mh_stride; a.sep_corr = 0;
+  a.n_tile = p.n_tile; a.chains = p.chains; a.mh_stride = p.mh_stride;
   a.kc = p.kc; a.stage_rows = p.stage_rows; a.raw_stride = p.raw_stride; a.t_slots = p.t_slots; a.tmem_cols = p.tmem_cols;
   a.chains = std::min(p.chains, (a.ci / p.kc) * a.k);          // never more chains than weight units
   if (p.chains > 2) throw std::runtime_error("conv2: at most two K-chains (the kernel picks the chain by comparison)");

@@ -1,7 +1,7 @@
-// DEFAULT since round 2 (PIPER_B200_V2=0 selects conv_mma.cu).  CUDA instantiation of the second-generation persistent tensor-core
-// convolution: the body lives in conv2_body.inl (what changes against conv_mma.cu is described there), the primitives
-// in tc_policy_dev.cuh, plan / pack / argument fill in conv2_host.h.  The same body runs on a CPU model of the primitives
-// in tests/test_conv2_sim.py (every epilogue, both split precisions, ragged batches); on the B200: tests/test_gpu_conv_kernels.py and the whole -m gpu suite.
+// CUDA instantiation of the persistent tensor-core convolution that runs every dense conv layer the engine routes to the
+// tensor cores: the body lives in conv2_body.inl, the primitives in tc_policy_dev.cuh, plan / pack / argument fill in
+// conv2_host.h.  The same body runs on a CPU model of the primitives in tests/test_conv2_sim.py (every epilogue, every
+// split precision, ragged batches); on the B200: tests/test_gpu_conv_kernels.py and the whole -m gpu suite.
 #include "kernels.cuh"
 #include "launch.cuh"
 
@@ -102,8 +102,8 @@ void conv2_pack(const float* wsrc, int ci, int k, int rows_p, const Conv2Layer& 
 }
 
 // a: x / y / y2 / r / w (conv2_pack layout) / bias / len / shape / epilogue fields set by the caller
-bool launch_conv2(MmaConvArgs a, const Conv2Layer& l, int B, int max_len, cudaStream_t st) {
-  if (B <= 0 || max_len <= 0) return true;
+void launch_conv2(MmaConvArgs a, const Conv2Layer& l, int B, int max_len, cudaStream_t st) {
+  if (B <= 0 || max_len <= 0) return;
   const conv2::Plan p = to_plan(l);
   static int g_tm = -1;                                 // PIPER_B200_V2_TM: tensor-map TMA for the activation window
   if (g_tm < 0) {
@@ -136,12 +136,6 @@ bool launch_conv2(MmaConvArgs a, const Conv2Layer& l, int B, int max_len, cudaSt
   } else if (!tm && a.astat) {
     grid = conv2::fill_args(a, p, B, max_len, false, nullptr, false, &smem);   // (the A-stationary instantiations exist for the tensor-map kernel only)
   }
-  static int g_small_too = -1;                          // PIPER_B200_V2=2: also take launches with fewer tiles than SMs
-  if (g_small_too < 0) {
-    const char* e = std::getenv("PIPER_B200_V2");
-    g_small_too = (e ? std::atoi(e) >= 2 : true) ? 1 : 0;   // default: every launch (1 = only launches with >= 148 tiles)
-  }
-  if (a.total_tiles < 148 && !g_small_too) return false;   // small launches stay on the one-tile-per-CTA kernel
   static bool attr_set[64] = {};
   int dev = 0;
   cudaGetDevice(&dev);
@@ -171,7 +165,7 @@ bool launch_conv2(MmaConvArgs a, const Conv2Layer& l, int B, int max_len, cudaSt
     else if (p.mt == 256) launch_k(conv2_tm_kernel<0, 256, 0>, dim3(grid), dim3(conv2::C2_THREADS), sm, st, a, tmx);
     else launch_k(conv2_tm_kernel<0, 128, 0>, dim3(grid), dim3(conv2::C2_THREADS), sm, st, a, tmx);
     count_launch();
-    return true;
+    return;
   }
   if (tm) {
     const size_t sm = smem + 128;
@@ -181,7 +175,7 @@ bool launch_conv2(MmaConvArgs a, const Conv2Layer& l, int B, int max_len, cudaSt
     else if (p.mt == 256) launch_k(conv2_tm_kernel<0, 256>, dim3(grid), dim3(conv2::C2_THREADS), sm, st, a, tmx);
     else launch_k(conv2_tm_kernel<0, 128>, dim3(grid), dim3(conv2::C2_THREADS), sm, st, a, tmx);
     count_launch();
-    return true;
+    return;
   }
   if (p.prec == 1) launch_k(conv2_kernel<1, 128>, dim3(grid), dim3(conv2::C2_THREADS), smem, st, a);
   else if (p.prec == 2 && p.mt == 256) launch_k(conv2_kernel<2, 256>, dim3(grid), dim3(conv2::C2_THREADS), smem, st, a);
@@ -189,7 +183,6 @@ bool launch_conv2(MmaConvArgs a, const Conv2Layer& l, int B, int max_len, cudaSt
   else if (p.mt == 256) launch_k(conv2_kernel<0, 256>, dim3(grid), dim3(conv2::C2_THREADS), smem, st, a);
   else launch_k(conv2_kernel<0, 128>, dim3(grid), dim3(conv2::C2_THREADS), smem, st, a);
   count_launch();
-  return true;
 }
 
 }  // namespace pb200

@@ -40,148 +40,10 @@ constexpr int ATT_QPW = 4;
 constexpr int ATT_Q = 8 * ATT_QPW;
 constexpr int ATT_MAXR = 4;
 
-__global__ void __launch_bounds__(256) rel_attention_kernel(View qkv, View out, const float* __restrict__ rel_k,
-                                                            const float* __restrict__ rel_v, int H, int dk, int window,
-                                                            const int* __restrict__ len) {
-  pdl_launch_dependents();   // programmatic dependent launch (launch.cuh): the next grid may be scheduled now;
-  pdl_wait();                // nothing below runs before the previous grid has completed
-  extern __shared__ float sm[];
-  const int b = blockIdx.z, h = blockIdx.y;
-  const int T = len[b];
-  const int i0 = blockIdx.x * ATT_Q;
-  if (i0 >= T) return;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int nrel = 2 * window + 1;
-  float* Ks = sm;                       // [dk][33]
-  float* Vs = Ks + dk * 33;             // [dk][33]
-  float* Qs = Vs + dk * 33;             // [ATT_Q][dk]
-  float* Rl = Qs + ATT_Q * dk;          // [ATT_Q][nrel]   relative-key logits per query
-  float* Ev = Rl + ATT_Q * nrel;        // [nrel][dk]      emb_rel_v
-
-  const float* base = qkv.p + (long long)b * qkv.bs;
-  const float* qg = base + (long long)(h * dk) * qkv.cs;
-  const float* kg = base + (long long)(H + h * dk) * qkv.cs;
-  const float* vg = base + (long long)(2 * H + h * dk) * qkv.cs;
-
-  for (int idx = threadIdx.x; idx < ATT_Q * dk; idx += 256) {
-    const int d = idx / ATT_Q, qi = idx - d * ATT_Q;          // consecutive threads -> consecutive query positions
-    const int i = i0 + qi;
-    Qs[qi * dk + d] = i < T ? qg[(long long)d * qkv.cs + i] / sqrtf((float)dk) : 0.f;   // query / sqrt(k_channels), attentions.py:232
-  }
-  for (int idx = threadIdx.x; idx < nrel * dk; idx += 256) Ev[idx] = rel_v[idx];
-  __syncthreads();
-  // relative-key logits: Rl[qi][r] = q_i . emb_rel_k[r]
-#pragma unroll
-  for (int qq = 0; qq < ATT_QPW; ++qq) {
-    const int qi = warp * ATT_QPW + qq;
-    for (int r = 0; r < nrel; ++r) {
-      float p = 0.f;
-      for (int d = lane; d < dk; d += 32) p += Qs[qi * dk + d] * __ldg(rel_k + r * dk + d);
-      for (int o = 16; o; o >>= 1) p += __shfl_xor_sync(0xffffffffu, p, o);
-      if (lane == 0) Rl[qi * nrel + r] = p;
-    }
-  }
-  __syncwarp();
-
-  float m_run[ATT_QPW], l_run[ATT_QPW], acc[ATT_QPW][ATT_MAXR];
-#pragma unroll
-  for (int qq = 0; qq < ATT_QPW; ++qq) {
-    m_run[qq] = -INFINITY;
-    l_run[qq] = 0.f;
-#pragma unroll
-    for (int r = 0; r < ATT_MAXR; ++r) acc[qq][r] = 0.f;
-  }
-  const int iq0 = i0 + warp * ATT_QPW;            // first query row of this warp
-
-  for (int j0 = 0; j0 < T; j0 += 32) {
-    __syncthreads();  // previous chunk fully consumed
-    for (int idx = threadIdx.x; idx < dk * 32; idx += 256) {
-      const int d = idx >> 5, jj = idx & 31;
-      const int j = j0 + jj;
-      float kv = 0.f, vv = 0.f;
-      if (j < T) {
-        kv = kg[(long long)d * qkv.cs + j];
-        vv = vg[(long long)d * qkv.cs + j];
-      }
-      Ks[d * 33 + jj] = kv;
-      Vs[d * 33 + jj] = vv;
-    }
-    __syncthreads();
-    if (iq0 >= T) continue;                        // warp-uniform; the barriers above are still reached
-    const int j = j0 + lane;
-    const int jn = min(32, T - j0);
-    float s[ATT_QPW];
-#pragma unroll
-    for (int qq = 0; qq < ATT_QPW; ++qq) s[qq] = 0.f;
-    for (int d = 0; d < dk; ++d) {
-      const float kd = Ks[d * 33 + lane];
-#pragma unroll
-      for (int qq = 0; qq < ATT_QPW; ++qq) s[qq] = fmaf(Qs[(warp * ATT_QPW + qq) * dk + d], kd, s[qq]);
-    }
-    float p[ATT_QPW];
-#pragma unroll
-    for (int qq = 0; qq < ATT_QPW; ++qq) {
-      const int i = iq0 + qq;
-      float sc = s[qq];
-      const int rel = j - i + window;
-      if (rel >= 0 && rel < nrel) sc += Rl[(warp * ATT_QPW + qq) * nrel + rel];
-      if (j >= T || i >= T) sc = -INFINITY;   // keys past the utterance: masked_fill(-1e4) -> exp underflows to exactly 0
-      float cmax = sc;
-      for (int o = 16; o; o >>= 1) cmax = fmaxf(cmax, __shfl_xor_sync(0xffffffffu, cmax, o));
-      const float m_new = fmaxf(m_run[qq], cmax);
-      const float corr = (m_new == -INFINITY) ? 1.f : expf(m_run[qq] - m_new);
-      p[qq] = (m_new == -INFINITY) ? 0.f : expf(sc - m_new);
-      float psum = p[qq];
-      for (int o = 16; o; o >>= 1) psum += __shfl_xor_sync(0xffffffffu, psum, o);
-      l_run[qq] = l_run[qq] * corr + psum;
-#pragma unroll
-      for (int r = 0; r < ATT_MAXR; ++r) acc[qq][r] *= corr;
-      m_run[qq] = m_new;
-      // banded relative values: keys j with |j - i| <= window inside this chunk
-      const int jlo = max(j0, i - window), jhi = min(j0 + jn - 1, i + window);
-      for (int jb = jlo; jb <= jhi; ++jb) {
-        const float pj = __shfl_sync(0xffffffffu, p[qq], jb - j0);
-        const int relj = jb - i + window;
-#pragma unroll
-        for (int r = 0; r < ATT_MAXR; ++r) {
-          const int d = lane + 32 * r;
-          if (d < dk) acc[qq][r] = fmaf(pj, Ev[relj * dk + d], acc[qq][r]);
-        }
-      }
-    }
-    // P.V: one V read per (key, channel) shared by the warp's queries
-    for (int jj = 0; jj < jn; ++jj) {
-      float pj[ATT_QPW];
-#pragma unroll
-      for (int qq = 0; qq < ATT_QPW; ++qq) pj[qq] = __shfl_sync(0xffffffffu, p[qq], jj);
-#pragma unroll
-      for (int r = 0; r < ATT_MAXR; ++r) {
-        const int d = lane + 32 * r;
-        if (d < dk) {
-          const float v = Vs[d * 33 + jj];
-#pragma unroll
-          for (int qq = 0; qq < ATT_QPW; ++qq) acc[qq][r] = fmaf(pj[qq], v, acc[qq][r]);
-        }
-      }
-    }
-  }
-  float* ob = out.p + (long long)b * out.bs + (long long)(h * dk) * out.cs;
-#pragma unroll
-  for (int qq = 0; qq < ATT_QPW; ++qq) {
-    const int i = iq0 + qq;
-    if (i >= T) continue;
-#pragma unroll
-    for (int r = 0; r < ATT_MAXR; ++r) {
-      const int d = lane + 32 * r;
-      if (d < dk) ob[(long long)d * out.cs + i] = acc[qq][r] / l_run[qq];
-    }
-  }
-}
-
-// Second version of the CUDA-core kernel (PIPER_B200_ATT2, default 1; used when PIPER_B200_ATT3=0): the same kernel with the staged queries kept
-// per warp as [d][4 queries], so the score loop issues one K load and ONE 16-byte broadcast load per 4 FMAs instead of one
-// K load and four scalar broadcast loads - the loop is bound by the shared-memory pipe (DESIGN.md section 8).  Same
-// arithmetic in the same order as rel_attention_kernel.
+// CUDA-core attention: the fallback for shapes the tensor-core kernel (att_mma.cu) declines, and all of it under
+// PIPER_B200_ATT3=0.  The staged queries are kept per warp as [d][4 queries], so the score loop issues one K load and ONE
+// 16-byte broadcast load per 4 FMAs instead of one K load and four scalar broadcast loads - the loop is bound by the
+// shared-memory pipe (DESIGN.md section 8).
 static_assert(ATT_QPW == 4, "rel_attention_kernel2 packs the four queries of a warp into one float4");
 __global__ void __launch_bounds__(256) rel_attention_kernel2(View qkv, View out, const float* __restrict__ rel_k,
                                                             const float* __restrict__ rel_v, int H, int dk, int window,
@@ -492,77 +354,11 @@ __global__ void __launch_bounds__(256) rel_attention_tail_kernel(View qkv, View 
 
 __device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.f + erff(x * 0.70710678118654752440f)); }
 
-// LayerNorm over channels for a tile of 32 time steps; 8 warps split the channel axis.
-// Values are staged in shared memory [C][33] so the (optional) depthwise conv is evaluated once.
-__global__ void __launch_bounds__(256) layernorm_kernel(const LnArgs a) {
-  pdl_launch_dependents();   // programmatic dependent launch (launch.cuh): the next grid may be scheduled now;
-  pdl_wait();                // nothing below runs before the previous grid has completed
-  extern __shared__ float sm[];
-  __shared__ float red[8][32];
-  const int b = blockIdx.z;
-  const int T = a.len[b];
-  const int t0 = blockIdx.x * 32;
-  if (t0 >= T) return;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int t = t0 + lane;
-  const bool live = t < T;
-  const int C = a.C;
-  const float* ab = a.a.p + (long long)b * a.a.bs;
-
-  for (int c = warp; c < C; c += 8) {
-    float v = 0.f;
-    if (live) {
-      const float* ar = ab + (long long)c * a.a.cs;
-      if (a.mode == LN_DW_GELU) {
-        v = __ldg(a.dw_b + c);
-        const int half = (a.dw_k - 1) / 2;
-        for (int j = 0; j < a.dw_k; ++j) {
-          const int tt = t + (j - half) * a.dw_dil;
-          if (tt >= 0 && tt < T) v = fmaf(__ldg(a.dw_w + c * a.dw_k + j), ar[tt], v);
-        }
-      } else {
-        v = ar[t];
-        if (a.mode == LN_ADD) v += a.b.p[(long long)b * a.b.bs + (long long)c * a.b.cs + t];
-      }
-    }
-    sm[c * 33 + lane] = v;
-  }
-  __syncthreads();
-  float s = 0.f;
-  for (int c = warp; c < C; c += 8) s += sm[c * 33 + lane];
-  red[warp][lane] = s;
-  __syncthreads();
-  float mean = 0.f;
-#pragma unroll
-  for (int w = 0; w < 8; ++w) mean += red[w][lane];
-  mean /= (float)C;
-  __syncthreads();
-  float q = 0.f;
-  for (int c = warp; c < C; c += 8) {
-    const float d = sm[c * 33 + lane] - mean;
-    q = fmaf(d, d, q);
-  }
-  red[warp][lane] = q;
-  __syncthreads();
-  float var = 0.f;
-#pragma unroll
-  for (int w = 0; w < 8; ++w) var += red[w][lane];
-  var /= (float)C;
-  const float rstd = 1.f / sqrtf(var + 1e-5f);
-  if (!live) return;
-  float* yb = a.y.p + (long long)b * a.y.bs;
-  for (int c = warp; c < C; c += 8) {
-    float v = (sm[c * 33 + lane] - mean) * rstd * __ldg(a.gamma + c) + __ldg(a.beta + c);
-    if (a.mode == LN_GELU_RES || a.mode == LN_DW_GELU) v = gelu_erf(v);
-    if (a.mode == LN_GELU_RES) v += a.r.p[(long long)b * a.r.bs + (long long)c * a.r.cs + t];
-    yb[(long long)c * a.y.cs + t] = v;
-  }
-}
-
-// DEFAULT since round 2 (PIPER_B200_LN2=0 selects layernorm_kernel): same arithmetic as layernorm_kernel in the same
-// order, but every warp issues its global loads eight channel rows at a time before using any of them.  The shipped kernel
-// walks its 24 rows (C = 192) one dependent load -> store at a time in both passes, which is what its ~28 us per launch
-// (36 launches per step) looks like: ~2 x 24 exposed L2 / DRAM latencies with only 16 warps per SM to hide them.
+// LayerNorm over channels for a tile of 32 time steps; the warps split the channel axis.  Values are staged in shared
+// memory [C][33] so the (optional) depthwise conv is evaluated once.  Every warp issues its global loads eight channel rows
+// at a time before using any of them: walking 24 rows (C = 192) one dependent load -> store at a time in both passes
+// measured ~28 us per launch (36 launches per step), ~2 x 24 exposed L2 / DRAM latencies with only 16 warps per SM to
+// hide them.
 constexpr int LN_U = 8;
 // NW warps per CTA: 24 for C >= 96 (each warp then owns <= 8 channel rows: ONE batch of loads per pass instead of three)
 template <int NW>
@@ -696,18 +492,20 @@ void launch_rel_attention(View qkv, View out, const float* rel_k, const float* r
   if (dk > 32 * ATT_MAXR) throw std::runtime_error("attention: head width > 128 is not supported");
   const int nrel = 2 * window + 1;
   const size_t smem = size_t(2 * dk * 33 + ATT_Q * dk + ATT_Q * nrel + nrel * dk) * sizeof(float);
-  static bool attr_set[64] = {};
   int dev = 0;
   cudaGetDevice(&dev);
-  if (!attr_set[dev & 63]) {
-    cudaFuncSetAttribute(rel_attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-    attr_set[dev & 63] = true;
-  }
+  auto kernel2_attr = [dev] {        // set where the CUDA-core kernel runs: the default path never loads it
+    static bool attr_set[64] = {};
+    if (!attr_set[dev & 63]) {
+      cudaFuncSetAttribute(rel_attention_kernel2, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+      attr_set[dev & 63] = true;
+    }
+  };
   dim3 grid((Tmax + ATT_Q - 1) / ATT_Q, n_heads, B);
-  static int g_att3 = -1;                                 // experimental tensor-core attention (att_mma.cu)
+  static int g_att3 = -1;                                 // PIPER_B200_ATT3: tensor-core attention (att_mma.cu)
   if (g_att3 < 0) {
     const char* e = std::getenv("PIPER_B200_ATT3");
-    g_att3 = e ? std::atoi(e) : 1;                       // default since round 2: tcgen05 attention (0 = CUDA-core kernel)
+    g_att3 = e ? std::atoi(e) : 1;                       // default on (0 = CUDA-core kernel for every shape)
   }
   int tail_thr = 0;
   if (g_att3 && launch_rel_attention_tc(qkv, out, rel_k, rel_v, H, n_heads, window, len, B, Tmax, st, &tail_thr)) {
@@ -727,7 +525,7 @@ void launch_rel_attention(View qkv, View out, const float* rel_k, const float* r
         launch_k(rel_attention_tail_kernel, dim3((tail_thr + ATT_QPW - 1) / ATT_QPW, n_heads, B), dim3(256), smem_t, st, qkv, out,
                  rel_k, rel_v, H, dk, window, len, tail_thr, n_w);
       } else {
-        cudaFuncSetAttribute(rel_attention_kernel2, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+        kernel2_attr();
         launch_k(rel_attention_kernel2, dim3((tail_thr + ATT_Q - 1) / ATT_Q, n_heads, B), dim3(256), smem, st, qkv, out, rel_k, rel_v, H,
                  dk, window, len, tail_thr);
       }
@@ -735,14 +533,8 @@ void launch_rel_attention(View qkv, View out, const float* rel_k, const float* r
     }
     return;
   }
-  static int g_att2 = -1;
-  if (g_att2 < 0) {
-    const char* e = std::getenv("PIPER_B200_ATT2");
-    g_att2 = e ? std::atoi(e) : 1;                       // default since round 2 (measured +; 0 = first version)
-    if (g_att2) cudaFuncSetAttribute(rel_attention_kernel2, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-  }
-  if (g_att2) launch_k(rel_attention_kernel2, dim3(grid), dim3(256), smem, st, qkv, out, rel_k, rel_v, H, dk, window, len, 0);
-  else launch_k(rel_attention_kernel, dim3(grid), dim3(256), smem, st, qkv, out, rel_k, rel_v, H, dk, window, len);
+  kernel2_attr();
+  launch_k(rel_attention_kernel2, dim3(grid), dim3(256), smem, st, qkv, out, rel_k, rel_v, H, dk, window, len, 0);
   count_launch();
 }
 
@@ -754,19 +546,11 @@ void launch_layernorm(const LnArgs& a, int B, int Tmax, cudaStream_t st) {
   int dev = 0;
   cudaGetDevice(&dev);
   if (!attr_set[dev & 63]) {
-    cudaFuncSetAttribute(layernorm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+    cudaFuncSetAttribute(layernorm_kernel2<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+    cudaFuncSetAttribute(layernorm_kernel2<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
     attr_set[dev & 63] = true;
   }
   dim3 grid((Tmax + 31) / 32, 1, B);
-  static int g_ln2 = -1;                                  // experimental batched-load variant (see layernorm_kernel2)
-  if (g_ln2 < 0) {
-    const char* e = std::getenv("PIPER_B200_LN2");
-    g_ln2 = e ? std::atoi(e) : 1;                        // default since round 2 (0 = first version)
-    if (g_ln2) {
-      cudaFuncSetAttribute(layernorm_kernel2<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-      cudaFuncSetAttribute(layernorm_kernel2<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-    }
-  }
   static int g_ln_warps = -1;                             // PIPER_B200_LN_WARPS: 8 / 24 warps per CTA (default: by problem size)
   if (g_ln_warps < 0) {
     const char* e = std::getenv("PIPER_B200_LN_WARPS");
@@ -775,9 +559,8 @@ void launch_layernorm(const LnArgs& a, int B, int Tmax, cudaStream_t st) {
   // 24 warps (one batch of loads per pass) shorten a latency-bound launch; with several CTAs per SM already resident the
   // 8-warp form has the same loads in flight and less barrier traffic (measured: batch 1 prefers 24, batch 32 prefers 8)
   const bool wide = g_ln_warps ? g_ln_warps == 24 : (long long)grid.x * B <= 148;
-  if (g_ln2 && a.C >= 96 && wide) launch_k(layernorm_kernel2<24>, dim3(grid), dim3(24 * 32), smem, st, a);
-  else if (g_ln2) launch_k(layernorm_kernel2<8>, dim3(grid), dim3(256), smem, st, a);
-  else launch_k(layernorm_kernel, dim3(grid), dim3(256), smem, st, a);
+  if (a.C >= 96 && wide) launch_k(layernorm_kernel2<24>, dim3(grid), dim3(24 * 32), smem, st, a);
+  else launch_k(layernorm_kernel2<8>, dim3(grid), dim3(256), smem, st, a);
   count_launch();
 }
 

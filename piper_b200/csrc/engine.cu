@@ -88,11 +88,6 @@ Engine::Engine(const std::string& onnx_path, int device, bool upload) : device_(
   weights_.ensure(voice_.blob.size() * sizeof(float));
   if (upload)
     CUDA_CHECK(cudaMemcpyAsync(weights_.p, voice_.blob.data(), voice_.blob.size() * sizeof(float), cudaMemcpyHostToDevice, stream_));
-  if (!voice_.blob_mma.empty()) {
-    weights_mma_.ensure(voice_.blob_mma.size());
-    if (upload)
-      CUDA_CHECK(cudaMemcpyAsync(weights_mma_.p, voice_.blob_mma.data(), voice_.blob_mma.size(), cudaMemcpyHostToDevice, stream_));
-  }
   CUDA_CHECK(cudaStreamSynchronize(stream_));    // uploads from pageable memory: complete before the first kernel reads them
   if (const char* e = std::getenv("PIPER_B200_MMA")) mma_mask_ = std::atoi(e);
 }
@@ -101,11 +96,11 @@ Engine::~Engine() {
   cudaSetDevice(device_);
   if (stream_) cudaStreamSynchronize(stream_);
   drop_graphs();
-  DeviceBuf* dbs[] = {&weights_, &weights_mma_, &ids_d_, &len_d_, &ylen_d_, &cum_d_, &logw_d_, &override_d_, &epsdp_d_, &epsoff_d_,
+  DeviceBuf* dbs[] = {&weights_, &ids_d_, &len_d_, &ylen_d_, &cum_d_, &logw_d_, &override_d_, &epsdp_d_, &epsoff_d_,
                       &off_d_, &sid_d_, &cond_d_, &x_, &t1_, &qkv_, &att_, &ffn_, &stats_, &g_, &h_, &u_, &v_, &pr_, &z2_, &z_, &fh_,
                       &facts_, &fout_, &epsz_d_, &ga_, &gp_, &gq_, &gs_, &audio_d_, &audio16_d_, &peak_d_, &mrf_w_, &params_d_, &prof_d_};
   for (auto* d : dbs) d->release();
-  for (auto& kv : v2_layers_)
+  for (auto& kv : conv2_layers_)
     if (kv.second.w_dev) cudaFree(kv.second.w_dev);
   PinnedBuf* pbs[] = {&ids_pin_, &misc_pin_, &audio_pin_, &audio16_pin_, &eps_pin_, &params_pin_, &override_pin_};
   for (auto* p : pbs) p->release();
@@ -130,55 +125,45 @@ ConvArgs Engine::conv_args(const ConvW& c, View x, const int* len, int len_scale
 }
 
 void Engine::conv(const char* tag, ConvArgs& a, int max_len, double len_sum) {
-  // route through the tensor cores when the layer has a split-precision copy and its family is enabled
+  // the tensor cores when the layer's family is enabled in the mask and the conv2 plan takes its shape, CUDA cores otherwise
   const ConvW* w = a.host_w;
   const int family = tag[0] == 'd' && tag[1] == 'e' ? 1 : tag[0] == 'f' ? 2 : tag[0] == 'e' ? 4 : tag[0] == 'd' && tag[1] == 'p' ? 8 : 0;
-  const bool mma = w && w->mma >= 0 && (mma_mask_ & family);
-  MmaConvArgs m;
-  if (mma) {
+  const bool fp32_grade = family != 1;                 // flow, encoder, duration predictor: their outputs feed exp() / ceil()
+  const Conv2Layer* l = w && (mma_mask_ & family) ? conv2_layer(*w, a, fp32_grade) : nullptr;
+  if (l && fp32_grade) {
+    // a launch of the throughput plan that would leave most SMs idle takes the latency plan instead (batch 1)
+    const long long rows = a.x.bs < (long long)a.x.cs ? (long long)B_ * a.x.bs : (long long)B_ * max_len;
+    const long long ctas = (rows + l->mt - 1) / l->mt * l->n_tiles;
+    if (ctas < 74)
+      if (const Conv2Layer* l1 = conv2_layer(*w, a, fp32_grade, 1)) l = l1;
+  }
+  auto go = [&] {
+    if (!l) {
+      launch_conv1d(a, B_, max_len, stream_);
+      return;
+    }
+    MmaConvArgs m;
     m.x = a.x; m.y = a.y; m.y2 = a.y2; m.r = a.r;
-    m.w = weights_mma_.as<uint8_t>() + w->mma;
+    m.w = static_cast<const uint8_t*>(l->w_dev);
     m.bias = a.bias; m.bias_item = a.bias_item; m.bias_item_stride = a.bias_item_stride;
     m.len = a.len; m.len_scale = a.len_scale;
     m.ci = a.ci; m.rows = a.rows; m.k = a.k; m.dil = a.dil; m.pad = a.pad; m.q_extra = a.q_extra;
     m.pre = a.pre; m.slope = a.slope; m.epi = a.epi; m.split = a.split; m.first = a.first;
     m.up = a.up; m.up_pad = a.up_pad; m.mrf = a.mrf; m.mrf_n = a.mrf_n;
-  }
-  if (v2_ < 0) {
-    const char* e = std::getenv("PIPER_B200_V2");
-    v2_ = e ? std::atoi(e) : 2;                        // default since round 2: the second-generation kernel for every launch (0 = first generation)
-  }
-  auto go = [&] {
-    if (mma && v2_) {                                  // experimental kernel first; it declines small launches
-      const Conv2Layer* l = v2_layer(*w, a);
-      if (l && w->plan.tf32) {
-        // a launch of the throughput plan that would leave most SMs idle takes the latency plan instead (batch 1)
-        const long long rows = a.x.bs < (long long)a.x.cs ? (long long)B_ * a.x.bs : (long long)B_ * max_len;
-        const long long ctas = (rows + l->mt - 1) / l->mt * l->n_tiles;
-        if (ctas < 74)
-          if (const Conv2Layer* l1 = v2_layer(*w, a, 1)) l = l1;
-      }
-      if (l) {
-        MmaConvArgs m2 = m;
-        m2.w = static_cast<const uint8_t*>(l->w_dev);
-        if (profile_ && prof_d_.p && recs_.size() < kProfRecs)       // per-role wait counters of this launch (conv2_body.inl)
-          m2.prof = prof_d_.as<unsigned long long>() + 16 * recs_.size();
-        // flat layout views (bs = slot < cs): one launch item of length items x slot, tiles on the concatenated time axis
-        auto same_layout = [&](const View& v) { return v.p == nullptr || (v.bs == a.x.bs && v.cs == a.x.cs); };
-        const bool flat = flat_ > 0 && a.len_scale == 1 && a.q_extra == 0 && a.x.bs < (long long)a.x.cs && a.x.bs * B_ == a.x.cs &&
-                          a.x.bs >= 2 && ((long long)a.x.cs + 1024) * a.x.bs < (1LL << 32) &&   // (range of the kernel's reciprocal division)
-                          same_layout(a.y) && same_layout(a.y2) && same_layout(a.r);   // (conv_pre writes an item-major generator buffer)
-        if (flat) {
-          m2.flat_tg = int(a.x.bs);
-          m2.flat_n = B_;
-          if (launch_conv2(m2, *l, 1, B_ * int(a.x.bs), stream_)) return;
-          m2.flat_tg = m2.flat_n = 0;
-        }
-        if (launch_conv2(m2, *l, B_, max_len, stream_)) return;
-      }
+    if (profile_ && prof_d_.p && recs_.size() < kProfRecs)       // per-role wait counters of this launch (conv2_body.inl)
+      m.prof = prof_d_.as<unsigned long long>() + 16 * recs_.size();
+    // flat layout views (bs = slot < cs): one launch item of length items x slot, tiles on the concatenated time axis
+    auto same_layout = [&](const View& v) { return v.p == nullptr || (v.bs == a.x.bs && v.cs == a.x.cs); };
+    const bool flat = flat_ > 0 && a.len_scale == 1 && a.q_extra == 0 && a.x.bs < (long long)a.x.cs && a.x.bs * B_ == a.x.cs &&
+                      a.x.bs >= 2 && ((long long)a.x.cs + 1024) * a.x.bs < (1LL << 32) &&   // (range of the kernel's reciprocal division)
+                      same_layout(a.y) && same_layout(a.y2) && same_layout(a.r);   // (conv_pre writes an item-major generator buffer)
+    if (flat) {
+      m.flat_tg = int(a.x.bs);
+      m.flat_n = B_;
+      launch_conv2(m, *l, 1, B_ * int(a.x.bs), stream_);
+    } else {
+      launch_conv2(m, *l, B_, max_len, stream_);
     }
-    if (mma) launch_conv_mma(m, w->plan, B_, max_len, stream_);
-    else launch_conv1d(a, B_, max_len, stream_);
   };
   if (!profile_) {
     go();
@@ -191,7 +176,7 @@ void Engine::conv(const char* tag, ConvArgs& a, int max_len, double len_sum) {
   }
   ProfRec r;
   r.tag = tag;
-  r.mma = mma;
+  r.mma = l != nullptr;
   r.e0 = ev_pool_[ev_used_++];
   r.e1 = ev_pool_[ev_used_++];
   // algorithmic work of this launch (SURVEY.md §8d): fp32 in + out + weights once; elementwise ops free
@@ -207,18 +192,18 @@ void Engine::conv(const char* tag, ConvArgs& a, int max_len, double len_sum) {
 
 // variant 0: the throughput plan (one K-chain for short reductions -> 128-row output tiles); variant 1: the latency plan for
 // launches that cannot fill the machine (two chains everywhere -> 64-row output tiles, i.e. more, lighter CTAs).
-const Conv2Layer* Engine::v2_layer(const ConvW& w, const ConvArgs& a, int variant) {
-  auto it = v2_layers_.find({&w, variant});
-  if (it == v2_layers_.end()) {
+const Conv2Layer* Engine::conv2_layer(const ConvW& w, const ConvArgs& a, bool fp32_grade, int variant) {
+  auto it = conv2_layers_.find({&w, variant});
+  if (it == conv2_layers_.end()) {
     Conv2Layer l;
-    // precision: as the shipped path (bf16x3 generator, tf32x3 elsewhere) or, with PIPER_B200_V2_PREC=f16, fp16x3 for
-    // every family (tf32x3-class accuracy at bf16x3 instruction cost, conv2_body.inl); 2 K-chains where tf32x3 has them
+    // precision: fp16x3 for every family (tf32x3-class accuracy at bf16x3 instruction cost, conv2_body.inl) or, with
+    // PIPER_B200_V2_PREC=std, bf16x3 for the generator and tf32x3 for the fp32-grade families; 2 K-chains for the latter
     static int g_f16 = -1;
     if (g_f16 < 0) {
       const char* e = std::getenv("PIPER_B200_V2_PREC");
       g_f16 = (e ? std::string(e) == "f16" : true) ? 1 : 0;      // default fp16x3 (PIPER_B200_V2_PREC=std: bf16x3 generator, tf32x3 elsewhere)
     }
-    const int prec = g_f16 ? 2 : (w.plan.tf32 ? 1 : 0);
+    const int prec = g_f16 ? 2 : (fp32_grade ? 1 : 0);
     static int g_chains = -1;                            // PIPER_B200_V2_CHAINS: K-chains of the fp32-grade families (default 2)
     if (g_chains < 0) {
       const char* e = std::getenv("PIPER_B200_V2_CHAINS");
@@ -232,7 +217,7 @@ const Conv2Layer* Engine::v2_layer(const ConvW& w, const ConvArgs& a, int varian
       const char* e = std::getenv("PIPER_B200_V2_CHAIN_K");
       g_chain_k = e ? std::atoi(e) : 400;               // measured: +1.6 % on config 3; real-voice error 2.8e-4 -> <= 3.6e-4
     }
-    const int chains = (w.plan.tf32 && (variant == 1 || a.ci * a.k >= g_chain_k)) ? g_chains : 1;
+    const int chains = (fp32_grade && (variant == 1 || a.ci * a.k >= g_chain_k)) ? g_chains : 1;
     if (conv2_plan(a.ci, a.rows, a.k, a.dil, prec, chains, l)) {
       std::vector<uint8_t> host(l.w_bytes);
       conv2_pack(voice_.blob.data() + w.w, a.ci, a.k, a.rows_p, l, host.data());
@@ -243,7 +228,7 @@ const Conv2Layer* Engine::v2_layer(const ConvW& w, const ConvArgs& a, int varian
       CUDA_CHECK(cudaMemcpyAsync(l.w_dev, host.data(), l.w_bytes, cudaMemcpyHostToDevice, stream_));
       CUDA_CHECK(cudaStreamSynchronize(stream_));
     }
-    it = v2_layers_.emplace(std::make_pair(&w, variant), l).first;
+    it = conv2_layers_.emplace(std::make_pair(&w, variant), l).first;
   }
   return it->second.w_dev ? &it->second : nullptr;
 }
@@ -730,7 +715,7 @@ void Engine::run_generator() {
     if (debug_) save_tap("up" + std::to_string(st), A, ch, ylen_h_.data(), rate);
     if ((mma_mask_ & 16) && !mrf_ready_) prepare_mrf_fused();
     if ((mma_mask_ & 16) && mrf_plans_[st].ok) {
-      // experimental: the whole stage (all resblocks and the MRF average) in one launch
+      // the whole stage (all resblocks and the MRF average) in one launch
       MrfFusedArgs f;
       f.x = A; f.y = S; f.len = ylen; f.len_scale = rate; f.slope = 0.1f;
       f.w = mrf_w_.as<uint8_t>() + mrf_w_off_[st];
@@ -833,7 +818,7 @@ void Engine::prepare_mrf_fused() {
   }
   if (!host.empty()) {
     mrf_w_.ensure(host.size());
-    CUDA_CHECK(cudaMemcpyAsync(mrf_w_.p, host.data(), host.size(), cudaMemcpyHostToDevice, stream_));   // (see v2_layer)
+    CUDA_CHECK(cudaMemcpyAsync(mrf_w_.p, host.data(), host.size(), cudaMemcpyHostToDevice, stream_));   // (see conv2_layer)
     CUDA_CHECK(cudaStreamSynchronize(stream_));
   }
   mrf_ready_ = true;

@@ -57,7 +57,7 @@ struct HostTap {
 
 class Engine {
  public:
-  // upload = false: allocate the HBM weight buffers but leave them unfilled (a peer broadcasts into them)
+  // upload = false: allocate the HBM weight buffer but leave it unfilled (a peer broadcasts into it)
   Engine(const std::string& onnx_path, int device, bool upload = true);
   ~Engine();
   Engine(const Engine&) = delete;
@@ -67,10 +67,9 @@ class Engine {
   const PackedVoice& voice() const { return voice_; }
   int device() const { return device_; }
   int64_t weight_bytes() const { return int64_t(voice_.blob.size()) * 4; }
-  // device pointers of the two weight blobs (fp32 layout, split-precision tensor-core layout) for load-time broadcast
-  void weight_buffers(void** fp32, int64_t* fp32_bytes, void** mma, int64_t* mma_bytes) const {
+  // device pointer of the fp32 weight blob for load-time broadcast
+  void weight_buffers(void** fp32, int64_t* fp32_bytes) const {
     *fp32 = weights_.p; *fp32_bytes = int64_t(voice_.blob.size()) * 4;
-    *mma = weights_mma_.p; *mma_bytes = int64_t(voice_.blob_mma.size());
   }
 
   // ---- whole pipeline, host buffers in / host buffer out (the reference-facing call)
@@ -120,8 +119,8 @@ class Engine {
   void ensure_front(int B, int Tmax);
   void ensure_back(int B, int Fmax);
   void collect_stage_times();
-  // every dense conv goes through here: tensor-core path when the layer has a split-precision copy and its
-  // family (1 = generator, 2 = flow, 4 = text encoder, 8 = duration predictor) is enabled, CUDA-core kernel otherwise
+  // every dense conv goes through here: the tensor-core kernel (conv_mma2.cu) when the layer's family (1 = generator,
+  // 2 = flow, 4 = text encoder, 8 = duration predictor) is enabled and conv2_plan takes its shape, CUDA-core kernel otherwise
   void conv(const char* tag, ConvArgs& a, int max_len, double len_sum);
   void profile_begin();
   void save_tap(const std::string& name, View v, int C, const int* len_host, int scale);
@@ -140,19 +139,18 @@ class Engine {
   int device_ = 0;
   cudaStream_t stream_ = nullptr;
   cudaEvent_t ev_[8] = {};
-  DeviceBuf weights_, weights_mma_;
-  // experimental second-generation conv kernel (PIPER_B200_V2=1, conv_mma2.cu): per-layer plan + stacked weights, lazily
-  int v2_ = -1;
-  std::map<std::pair<const ConvW*, int>, Conv2Layer> v2_layers_;      // (layer, variant): see v2_layer
-  const Conv2Layer* v2_layer(const ConvW& w, const ConvArgs& a, int variant = 0);
-  // experimental fused MRF stage (mask bit 16, mrf_fused.cu): packed lazily on first use
+  DeviceBuf weights_;
+  // tensor-core conv (conv_mma2.cu): per-layer plan + stacked weights, packed lazily from the fp32 blob; null = not taken
+  std::map<std::pair<const ConvW*, int>, Conv2Layer> conv2_layers_;   // (layer, variant): see conv2_layer
+  const Conv2Layer* conv2_layer(const ConvW& w, const ConvArgs& a, bool fp32_grade, int variant = 0);
+  // fused MRF stage (mask bit 16, mrf_fused.cu): packed lazily on first use
   void prepare_mrf_fused();
   bool mrf_ready_ = false;
   std::vector<MrfFusedPlan> mrf_plans_;
   MrfFusedPlan mrf_plan_post_;        // last stage with conv_post + tanh fused behind it (used when taps are off)
   std::vector<size_t> mrf_w_off_, mrf_b_off_;
   DeviceBuf mrf_w_;
-  int mma_mask_ = 31;  // generator bf16x3; flow, encoder, duration predictor tf32x3 with chained accumulators (DESIGN.md §3)
+  int mma_mask_ = 31;  // every conv family and the fused MRF stage on the tensor cores, fp16x3 (DESIGN.md §3)
 
   // request state
   int B_ = 0, Tmax_ = 0, Tp_ = 0, Fmax_ = 0, Fp_ = 0;

@@ -71,10 +71,10 @@ struct TmapDesc {
 // CUtensorMap (128 bytes, 64-byte aligned) from a TmapDesc through cuTensorMapEncodeTiled; false = the driver refused it.
 bool encode_tmap(const TmapDesc& d, void* out_cutensormap);
 
-// ---- tensor-core (tcgen05) Conv1d / ConvTranspose1d with split precision (conv_mma.cu) ----------------------
+// ---- persistent tensor-core (tcgen05) Conv1d / ConvTranspose1d with split precision (conv_mma2.cu) -------------
 struct MmaConvArgs {
   View x, y, y2, r;
-  const uint8_t* w = nullptr;    // packed by pack_conv_mma
+  const uint8_t* w = nullptr;    // packed by conv2_pack
   const float* bias = nullptr;
   const float* bias_item = nullptr;   // optional per-item bias (speaker conditioning)
   int bias_item_stride = 0;
@@ -85,9 +85,9 @@ struct MmaConvArgs {
   float slope = 0.f;
   int epi = EPI_BIAS;
   int split = 0, first = 0, up = 1, up_pad = 0, mrf = 0, mrf_n = 1;
-  int kc = 0, stage_rows = 0, n_tile = 0, acc_cols = 0, tmem_cols = 0, a_slots = 1, w_slots = 2;   // from the MmaPlan
-  int chains = 1, sep_corr = 0, mh_stride = 0;
-  int raw_stride = 0, tiles_per_item = 0, total_tiles = 0, batch = 0, t_slots = 1, tpu = 1;   // persistent kernel
+  int kc = 0, stage_rows = 0, n_tile = 0, tmem_cols = 0, a_slots = 1;   // from the Conv2Layer plan
+  int chains = 1, mh_stride = 0;
+  int raw_stride = 0, tiles_per_item = 0, total_tiles = 0, batch = 0, t_slots = 1;
   int tm_boxes = 0;              // conv2 tensor-map mode: boxes per channel chunk (0 = per-row bulk copies)
   int mma3 = 0;                  // conv2: three instructions per k-step on exactly matching accumulator regions (see conv2_body.inl)
   // conv2 flat mode: the views are laid out [channel][item][slot of flat_tg floats] (View.bs = flat_tg, View.cs = items *
@@ -100,10 +100,7 @@ struct MmaConvArgs {
   int astat = 0, n_tiles = 1;
   unsigned long long* prof = nullptr;   // optional: per-role stall cycle counters (tools/conv_diag.py)
 };
-void launch_conv_mma(MmaConvArgs a, const MmaPlan& p, int B, int max_len, cudaStream_t st);
-void run_mma_bench(int N, int tf32, int n_acc, int iters, int shift, unsigned long long out[2]);
 
-// ---- second-generation persistent tensor-core conv (conv_mma2.cu; default since round 2, PIPER_B200_V2=0 = first generation) ----
 struct Conv2Layer {          // tiling of one layer + where its stacked weights live (filled lazily by the engine)
   bool tf32 = false;
   int prec = 0;              // 0 bf16x3, 1 tf32x3, 2 fp16x3 (conv2_body.inl)
@@ -113,8 +110,7 @@ struct Conv2Layer {          // tiling of one layer + where its stacked weights 
 };
 bool conv2_plan(int ci, int rows, int k, int dil, int prec, int chains, Conv2Layer& l);
 void conv2_pack(const float* wsrc, int ci, int k, int rows_p, const Conv2Layer& l, uint8_t* out);
-// false: the launch is too small for the persistent kernel (caller falls back to launch_conv_mma)
-bool launch_conv2(MmaConvArgs a, const Conv2Layer& l, int B, int max_len, cudaStream_t st);
+void launch_conv2(MmaConvArgs a, const Conv2Layer& l, int B, int max_len, cudaStream_t st);
 
 // ---- one whole MRF stage (three resblocks) of the generator per launch (mrf_fused.cu; default for 32-channel stages) ----
 constexpr int MRF_MAX_CHAINS = 3, MRF_MAX_STEPS = 6;

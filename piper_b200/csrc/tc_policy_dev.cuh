@@ -1,5 +1,5 @@
 // Device implementation of the primitive policy the policy-based kernel bodies (mrf_fused_body.inl, conv2_body.inl) are
-// written against: inline PTX for tcgen05 / TMA / mbarrier, in the same forms conv_mma.cu has exercised on hardware.
+// written against: inline PTX for tcgen05 / TMA / mbarrier.
 // The CPU counterpart (a functional model used by tests) is tests/sim/sim_prim.h.
 #pragma once
 #include <cuda.h>
@@ -12,7 +12,7 @@
 namespace pb200 {
 namespace {
 
-// ---- tcgen05 / TMA / mbarrier primitives (same forms as conv_mma.cu, where they have been exercised on hardware) ----
+// ---- tcgen05 / TMA / mbarrier primitives -------------------------------------------------------------------------
 struct DevPrim {
   static constexpr bool kSim = false;
   using Mbar = uint64_t;
@@ -54,7 +54,7 @@ struct DevPrim {
   static __device__ __forceinline__ void mbar_expect_tx(Ctx& c, Mbar* m, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(saddr(c, m)), "r"(bytes) : "memory");
   }
-  // bounded: this kernel is experimental - a protocol bug must end as a trap (launch failure), not as a hung GPU
+  // bounded: a protocol bug must end as a trap (launch failure), not as a hung GPU
   static __device__ __forceinline__ void mbar_wait(Ctx& c, Mbar* m, uint32_t parity) {
     const uint32_t a = saddr(c, m);
     const long long t0 = clock64();

@@ -4,7 +4,6 @@
 #include "kernels.cuh"
 #include "launch.cuh"
 
-#include <cstdlib>
 #include <stdexcept>
 
 namespace pb200 {
@@ -15,45 +14,8 @@ namespace {
 constexpr int POST_TT = 256;
 constexpr int POST_MAXK = 15;
 
-__global__ void __launch_bounds__(256) conv_post_kernel(View x, const float* __restrict__ w, int C, int k, float slope,
-                                                        float* __restrict__ out, const long long* __restrict__ out_off,
-                                                        const int* __restrict__ len, int len_scale) {
-  pdl_launch_dependents();   // programmatic dependent launch (launch.cuh): the next grid may be scheduled now;
-  pdl_wait();                // nothing below runs before the previous grid has completed
-  extern __shared__ float sm[];   // weights [C][k] | activated input tile [C][POST_TT + k - 1]
-  const int b = blockIdx.z;
-  const int L = len[b] * len_scale;
-  const int t0 = blockIdx.x * POST_TT;
-  if (t0 >= L) return;
-  const int half = (k - 1) / 2;
-  const int span = POST_TT + k - 1;
-  float* ws = sm;
-  float* xs = sm + C * k;
-  for (int i = threadIdx.x; i < C * k; i += 256) ws[i] = w[i];
-  const float* xb = x.p + (long long)b * x.bs;
-  for (int c = 0; c < C; ++c) {                       // coalesced rows, leaky-relu applied once per element
-    const float* xr = xb + (long long)c * x.cs;
-    for (int u = threadIdx.x; u < span; u += 256) {
-      const int tt = t0 - half + u;
-      float v = (tt >= 0 && tt < L) ? __ldg(xr + tt) : 0.f;
-      xs[c * span + u] = v > 0.f ? v : v * slope;
-    }
-  }
-  __syncthreads();
-  const int t = t0 + threadIdx.x;
-  if (t >= L) return;
-  float acc = 0.f;
-  for (int c = 0; c < C; ++c) {
-    const float* xr = xs + c * span + threadIdx.x;
-    const float* wr = ws + c * k;
-    for (int j = 0; j < k; ++j) acc = fmaf(wr[j], xr[j], acc);
-  }
-  out[out_off[b] + t] = tanhf(acc);
-}
-
-// DEFAULT since round 2 where the fused MRF stage does not apply (PIPER_B200_POST2=0 selects conv_post_kernel): the same computation in the same order, with the
-// staging loads of eight channels in flight at once.  The shipped kernel stages its C = 32 rows one exposed load latency
-// after the other (~0.58 ms per step for 0.5 GB, 7x the HBM time).
+// conv_post where the fused MRF stage does not apply.  The staging loads of eight channels are in flight at once: staging
+// the C = 32 rows one exposed load latency after the other measured ~0.58 ms per step for 0.5 GB, 7x the HBM time.
 __global__ void __launch_bounds__(256) conv_post_kernel2(View x, const float* __restrict__ w, int C, int k, float slope,
                                                          float* __restrict__ out, const long long* __restrict__ out_off,
                                                          const int* __restrict__ len, int len_scale) {
@@ -140,17 +102,10 @@ void launch_conv_post(View x, const float* w, int C, int k, float slope, float* 
   int dev = 0;
   cudaGetDevice(&dev);
   if (!attr_set[dev & 63]) {
-    cudaFuncSetAttribute(conv_post_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+    cudaFuncSetAttribute(conv_post_kernel2, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
     attr_set[dev & 63] = true;
   }
-  static int g_post2 = -1;                                // experimental batched-load variant (see conv_post_kernel2)
-  if (g_post2 < 0) {
-    const char* e = std::getenv("PIPER_B200_POST2");   // default on since round 2
-    g_post2 = e ? std::atoi(e) : 1;
-    if (g_post2) cudaFuncSetAttribute(conv_post_kernel2, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-  }
-  if (g_post2) launch_k(conv_post_kernel2, dim3(grid), dim3(256), smem, st, x, w, C, k, slope, out, out_off, len, len_scale);
-  else launch_k(conv_post_kernel, dim3(grid), dim3(256), smem, st, x, w, C, k, slope, out, out_off, len, len_scale);
+  launch_k(conv_post_kernel2, dim3(grid), dim3(256), smem, st, x, w, C, k, slope, out, out_off, len, len_scale);
   count_launch();
 }
 

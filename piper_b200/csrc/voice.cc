@@ -196,19 +196,6 @@ struct Packer {
     return r;
   }
 
-  // split-precision copy for the tcgen05 path, built from the already packed fp32 [ci][k][rows_p] layout
-  void add_mma(ConvW& c, bool tf32) {
-    MmaPlan p;
-    if (c.w < 0 || !mma_plan(c.ci, c.rows, c.k, c.dil, tf32, p)) return;
-    std::vector<uint8_t> packed;
-    pack_conv_mma(&v.blob[size_t(c.w)], c.ci, c.k, c.rows, c.rows_p, p, packed);
-    const size_t off = (v.blob_mma.size() + 127) / 128 * 128;
-    v.blob_mma.resize(off + packed.size(), 0);
-    std::memcpy(&v.blob_mma[off], packed.data(), packed.size());
-    c.mma = int64_t(off);
-    c.plan = p;
-  }
-
   LayerNormW ln(const std::string& prefix, int c_expected) {
     LayerNormW r;
     const OnnxTensor& g = get(prefix + ".gamma", 1);
@@ -482,28 +469,6 @@ void load_voice_file(const std::string& onnx_path, PackedVoice& v) {
     }
   }
 
-  // ---- tensor-core copies: bf16x3 for the generator, tf32x3 where outputs feed exp()/ceil() (flow, encoder)
-  for (EncLayerW& e : v.enc) { P.add_mma(e.qkv, true); P.add_mma(e.o, true); P.add_mma(e.ffn1, true); P.add_mma(e.ffn2, true); }
-  P.add_mma(v.enc_proj, true);
-  for (CouplingW& cw : v.flow) {
-    P.add_mma(cw.pre, true);
-    P.add_mma(cw.post, true);
-    for (ConvW& c : cw.in_layers) P.add_mma(c, true);
-    for (ConvW& c : cw.res_skip) P.add_mma(c, true);
-  }
-  // duration predictor 1x1 convs (their output feeds exp()/ceil(): tf32x3)
-  P.add_mma(v.dp_pre, true);
-  P.add_mma(v.dp_proj, true);
-  for (DDSLayerW& l : v.dp_dds.layers) P.add_mma(l.pw, true);
-  for (ConvFlowW& cf : v.dp_flows)
-    for (DDSLayerW& l : cf.dds.layers) P.add_mma(l.pw, true);
-  P.add_mma(v.dec_pre, false);
-  for (ConvW& u : v.ups) P.add_mma(u, false);
-  for (auto& stage : v.resblocks)
-    for (ResBlockW& rb : stage) {
-      for (ConvW& c : rb.c1) P.add_mma(c, false);
-      for (ConvW& c : rb.c2) P.add_mma(c, false);
-    }
   // pad the tail so 16-byte vector loads of the last rows never leave the allocation
   v.blob.resize((v.blob.size() + 63) / 64 * 64 + 64, 0.f);
 }

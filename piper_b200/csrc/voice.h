@@ -14,15 +14,6 @@
 
 namespace pb200 {
 
-// Tiling of one layer on the tensor-core path (conv_mma.cu)
-struct MmaPlan {
-  bool tf32 = false;
-  int mt = 0, kc = 0, stage_rows = 0, n_tile = 0, n_tiles = 0, acc_cols = 0, tmem_cols = 0, a_slots = 1, w_slots = 2;
-  int chains = 1, mh_stride = 0;   // K-chains accumulated separately; TMEM columns per row half
-  bool sep_corr = false;           // hi*lo / lo*hi terms in their own accumulator
-  size_t smem = 0;
-};
-
 // A Conv1d / ConvTranspose1d lowered to "rows x (Ci*K)" with weights stored [Ci][K][RowsP]
 // (row index fastest) so a CTA's row tile is one contiguous, 16B-aligned run per (ci, tap).
 struct ConvW {
@@ -30,9 +21,6 @@ struct ConvW {
   int ci = 0, rows = 0, rows_p = 0, k = 1, dil = 1, pad = 0;
   // ConvTranspose lowering: rows = Co * up, output t = q*up + (row % up) - up_pad
   int up = 1, up_pad = 0;
-  // tensor-core copy (split-precision hi/lo units, see conv_mma.cu): byte offset into blob_mma, -1 if none
-  int64_t mma = -1;
-  MmaPlan plan;
 };
 
 struct LayerNormW {
@@ -85,7 +73,6 @@ struct VoiceSpec {
 struct PackedVoice {
   VoiceSpec spec;
   std::vector<float> blob;
-  std::vector<uint8_t> blob_mma;  // split-precision (bf16x3 / tf32x3) weight units for the tensor-core path
   int64_t emb = -1;
   std::vector<EncLayerW> enc;
   ConvW enc_proj;
@@ -112,10 +99,5 @@ void load_voice_file(const std::string& onnx_path, PackedVoice& out);
 
 // Human/test-readable description (JSON) of the inferred spec and packed layout.
 std::string describe_voice(const PackedVoice& v);
-
-// defined in conv_mma.cu (declared here so the host-only loader can call them)
-bool mma_plan(int ci, int rows, int k, int dil, bool tf32, MmaPlan& p);
-void pack_conv_mma(const float* wsrc /*[ci][k][rows_p]*/, int ci, int k, int rows, int rows_p, const MmaPlan& p,
-                   std::vector<uint8_t>& out);
 
 }  // namespace pb200

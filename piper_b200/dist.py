@@ -2,7 +2,8 @@
 hot path.  torch.distributed is used for exactly two things:
 
 * `load_voice_broadcast` — rank 0 uploads the packed weights, every other rank receives them with an NCCL
-  broadcast over NVLink / NVSwitch straight into the engine's HBM buffers (62.6 MB medium, 113 MB high);
+  broadcast over NVLink / NVSwitch straight into the engine's HBM buffer (62.6 MB medium, 113 MB high); the
+  tensor-core weights are packed by every rank from its own host parse of the voice;
 * `synthesize_sharded`   — optional gather of the per-rank results to rank 0 in input order (objects; works on
   gloo too, which is how the CPU test exercises the host logic without a GPU).
 """
@@ -24,17 +25,15 @@ class _DeviceBytes:
 
 
 def load_voice_broadcast(onnx_path: str, device: int, rank: int, src: int = 0):
-    """Load a voice on this rank's GPU; only `src` pays the H2D upload, the rest get the blobs over NCCL."""
+    """Load a voice on this rank's GPU; only `src` pays the H2D upload, the rest get the weights over NCCL."""
     import torch
     import torch.distributed as dist
     from . import engine
     voice = engine.Voice(onnx_path, device, upload=(rank == src))
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        for ptr, nbytes in voice.weight_buffers():
-            if not ptr or nbytes <= 0:
-                continue
-            t = torch.as_tensor(_DeviceBytes(ptr, nbytes), device=torch.device("cuda", device))
-            dist.broadcast(t, src=src)
+        ptr, nbytes = voice.weight_buffers()
+        t = torch.as_tensor(_DeviceBytes(ptr, nbytes), device=torch.device("cuda", device))
+        dist.broadcast(t, src=src)
         torch.cuda.synchronize(device)
     return voice
 

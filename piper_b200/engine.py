@@ -203,11 +203,11 @@ class Voice:
         return list(ms)
 
     def weight_buffers(self):
-        """[(device pointer, bytes)] of the fp32 blob and the tensor-core blob (for the load-time NCCL broadcast)."""
-        p0, p1 = C.c_void_p(), C.c_void_p()
-        n0, n1 = C.c_int64(0), C.c_int64(0)
-        check(self._lib.pb200_voice_weight_buffers(self._h, C.byref(p0), C.byref(n0), C.byref(p1), C.byref(n1)))
-        return [(p0.value, n0.value), (p1.value, n1.value)]
+        """(device pointer, bytes) of the fp32 weight blob (for the load-time NCCL broadcast)."""
+        p = C.c_void_p()
+        n = C.c_int64(0)
+        check(self._lib.pb200_voice_weight_buffers(self._h, C.byref(p), C.byref(n)))
+        return p.value, n.value
 
     def set_speakers(self, sids):
         """Speaker ids for the following calls (item b uses sids[min(b, len-1)]); empty -> speaker 0."""

@@ -191,9 +191,33 @@ def _piper_layer_shapes():
         out.add((C_, C_ // 2 * r, ku // r, 1, False))          # ConvTranspose lowered to stride-phase rows
     for C_ in (256, 128, 64, 32):
         for k, ds in ((3, (1, 2)), (5, (2, 6)), (7, (3, 12)), (3, (1, 3, 5)), (7, (1, 3, 5)), (11, (1, 3, 5))):
-            for d in ds:
+            for d in set(ds) | {1}:
                 out.add((C_, C_, k, d, False))
     return sorted(out)
+
+
+def _engine_plans(ci, k, tf32):
+    """(prec, chains) the engine plans a layer with (engine.cu conv2_layer): fp16x3 by default - 1 chain for the
+    generator; for the fp32-grade families 2 chains when ci * k >= 400 (1 otherwise) plus the 2-chain latency variant -
+    and, under PIPER_B200_V2_PREC=std, bf16x3 with 1 chain for the generator and tf32x3 with 2 chains elsewhere."""
+    if not tf32:
+        return [(2, 1), (0, 1)]
+    return sorted({(2, 2 if ci * k >= 400 else 1), (2, 2), (1, 2 if ci * k >= 400 else 1), (1, 2)})
+
+
+def _check_plan(info, ci, rows, k, dil, prec, want_chains):
+    ok, n_tile, n_tiles, mt, kc, stage_rows, raw_stride, t_slots, tmem_cols, chains, mh_stride, smem, w_bytes = list(info)
+    assert ok, (ci, rows, k, dil, prec, want_chains)
+    es, kstep = (4, 8) if prec == 1 else (2, 16)
+    assert mt in (128, 256) and (mt == 128 or (prec != 1 and chains == 1))          # 256-row tiles: 1-chain bf16 / fp16 only
+    assert n_tile * n_tiles == rows and n_tile % 16 == 0 and 2 * n_tile <= 256       # stacked instruction: N' = 2N <= 256
+    assert chains == want_chains and mh_stride == chains * 2 * n_tile
+    assert t_slots * (mt // 128) * mh_stride <= tmem_cols <= 512
+    assert ci % kc == 0 and kc % kstep == 0
+    assert stage_rows >= mt + (k - 1) * dil and stage_rows % 8 == 0 and raw_stride >= stage_rows + 4
+    assert smem == 2 * kc * raw_stride * 4 + 2 * 2 * kc * stage_rows * es + 4 * kc * 2 * n_tile * es <= 196 * 1024
+    assert (kc * raw_stride * 4) % 128 == 0 and (kc * stage_rows * es) % 128 == 0     # ring slots stay 128-byte aligned
+    assert w_bytes == rows * k * ci * 2 * es
 
 
 def test_plan_respects_hardware_limits_for_every_piper_layer(sim):
@@ -201,17 +225,32 @@ def test_plan_respects_hardware_limits_for_every_piper_layer(sim):
     info = (C.c_longlong * 13)()
     for ci, rows, k, dil, tf32 in _piper_layer_shapes():
         sim.conv2_sim_plan(ci, rows, k, dil, int(tf32), 2 if tf32 else 1, info)
-        ok, n_tile, n_tiles, mt, kc, stage_rows, raw_stride, t_slots, tmem_cols, chains, mh_stride, smem, w_bytes = list(info)
-        assert ok, (ci, rows, k, dil, tf32)
-        es, kstep = (4, 8) if tf32 else (2, 16)
-        assert n_tile * n_tiles == rows and n_tile % 16 == 0 and 2 * n_tile <= 256       # stacked instruction: N' = 2N <= 256
-        assert chains == (2 if tf32 else 1) and mh_stride == chains * 2 * n_tile
-        assert t_slots * (mt // 128) * mh_stride <= tmem_cols <= 512
-        assert ci % kc == 0 and kc % kstep == 0
-        assert stage_rows >= mt + (k - 1) * dil and stage_rows % 8 == 0 and raw_stride >= stage_rows + 4
-        assert smem == 2 * kc * raw_stride * 4 + 2 * 2 * kc * stage_rows * es + 4 * kc * 2 * n_tile * es <= 196 * 1024
-        assert (kc * raw_stride * 4) % 128 == 0 and (kc * stage_rows * es) % 128 == 0     # ring slots stay 128-byte aligned
-        assert w_bytes == rows * k * ci * 2 * es
+        _check_plan(info, ci, rows, k, dil, int(tf32), 2 if tf32 else 1)
+
+
+def _engine_plans(ci, k, tf32):
+    """(prec, chains) the engine plans a layer with (engine.cu conv2_layer): fp16x3 by default - 1 chain for the
+    generator; for the fp32-grade families 2 chains when ci * k >= 400 (1 otherwise) plus the 2-chain latency variant -
+    and, under PIPER_B200_V2_PREC=std, bf16x3 with 1 chain for the generator and tf32x3 with 2 chains elsewhere."""
+    if not tf32:
+        return [(2, 1), (0, 1)]
+    return sorted({(2, 2 if ci * k >= 400 else 1), (2, 2), (1, 2 if ci * k >= 400 else 1), (1, 2)})
+
+
+def test_tensor_core_plans_respect_hardware_limits(sim):
+    """Every dense layer shape of the x-low / medium / high presets gets a tensor-core tiling that fits the SM for every
+    precision and K-chain count the engine plans it with; shapes the plan declines stay on the CUDA-core kernel."""
+    sim.conv2_sim_plan.argtypes = [C.c_int] * 6 + [C.POINTER(C.c_longlong)]
+    info = (C.c_longlong * 13)()
+    for ci, rows, k, dil, tf32 in _piper_layer_shapes():
+        for prec, chains in _engine_plans(ci, k, tf32):
+            sim.conv2_sim_plan(ci, rows, k, dil, prec, chains, info)
+            _check_plan(info, ci, rows, k, dil, prec, chains)
+    for ci, rows, k, dil in ((192, 29, 1, 1), (1, 192, 1, 1), (100, 64, 3, 1)):
+        for tf32 in (False, True):
+            for prec, chains in _engine_plans(ci, k, tf32):
+                sim.conv2_sim_plan(ci, rows, k, dil, prec, chains, info)
+                assert info[0] == 0, (ci, rows, k, dil, prec, chains)
 
 
 @pytest.mark.parametrize("ci,rows,k,dil,tf32,epi", [(192, 384, 5, 1, True, "GATE"),     # flow in_layer: 128-wide tiles, one TMEM set

@@ -1,5 +1,6 @@
-"""Kernel-level GPU tests: the CUDA-core (backend 0) and tensor-core (tcgen05; 1 = bf16x3, 2 = tf32x3) Conv1d
-kernels against a float64 torch reference of the same op."""
+"""Kernel-level GPU tests: the CUDA-core (backend 0) and tensor-core (tcgen05, conv_mma2.cu; 1 = bf16x3, 2 = tf32x3 with
+2 K-chains, 5 = fp16x3 with 1 chain, 6 = fp16x3 with 2 chains) Conv1d kernels against a float64 torch reference of the
+same op.  (Backends 3 and 4 are the same kernels as 1 and 2.)"""
 import numpy as np
 import pytest
 
@@ -27,14 +28,14 @@ CASES = [  # (B, ci, co, k, dil, L)   every generator resblock shape of the medi
     (2, 192, 384, 5, 1, 519), (1, 192, 768, 3, 1, 259), (1, 768, 192, 3, 1, 259), (2, 96, 192, 1, 1, 600),
     (1, 192, 96, 1, 1, 333), (1, 48, 96, 1, 1, 150), (1, 192, 576, 1, 1, 259), (1, 96, 48, 1, 1, 257),
     (1, 192, 256, 7, 1, 519),
-    # enough tiles for the persistent, fully pipelined tensor-core kernel (>= 2 tiles per SM)
+    # enough tiles for every SM to walk several tiles of the persistent tensor-core kernel
     (4, 32, 32, 7, 12, 40000), (2, 64, 64, 5, 6, 45001), (2, 128, 128, 7, 3, 20003), (2, 192, 384, 5, 1, 6001),
     (1, 192, 768, 3, 1, 5000), (2, 256, 256, 3, 1, 9999),
 ]
 
 
 @pytest.mark.parametrize("case", CASES)
-@pytest.mark.parametrize("backend", [0, 1, 2])
+@pytest.mark.parametrize("backend", [0, 1, 2, 5, 6])
 def test_conv1d_kernels(lib_built, backend, case):
     from piper_b200 import engine
     B, ci, co, k, dil, L = case
@@ -46,7 +47,7 @@ def test_conv1d_kernels(lib_built, backend, case):
     ref = _ref(x, w, b, dil, 0.1, resid)
     y = engine.debug_conv1d(backend, x, w, b, dil, 0.1, resid)
     err = np.abs(y - ref).max()
-    # fp32 FFMA / tf32x3: accumulation-order noise; bf16x3: ~2^-16 relative per product on O(1) outputs
+    # fp32 FFMA / tf32x3 / fp16x3: accumulation-order noise; bf16x3: ~2^-16 relative per product on O(1) outputs
     tol = 3e-4 if backend else 1e-4      # tensor-core fp32 accumulation truncates (RZ): error grows ~linearly with K
     assert err <= tol, err
     y2 = engine.debug_conv1d(backend, x, w, None, dil, 0.0, None)

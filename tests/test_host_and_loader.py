@@ -229,43 +229,6 @@ def test_shard_utterances_balanced_and_complete():
         assert max(loads) - min(loads) <= max(lens)
 
 
-def test_tensor_core_plans_respect_hardware_limits(lib_built):
-    """Every dense layer shape of the x-low / medium / high presets gets a tensor-core tiling that fits the SM:
-    <= 227 KB shared memory, <= 512 TMEM columns, chunk divides C_in, row tiles are multiples of 16 and <= 256."""
-    import ctypes as C
-    from piper_b200._lib import check
-    shapes = set()
-    for H, F in ((96, 384), (192, 768)):                     # text encoder / flow / duration predictor (tf32x3)
-        for ci, rows, k in ((H, 3 * H, 1), (H, H, 1), (H, F, 3), (F, H, 3), (H, 2 * H, 1), (H // 2, H, 1),
-                            (H, 2 * H, 5), (H, H // 2, 1)):
-            shapes.add((ci, rows, k, 1, 1))
-    for C0, ups, ks, dils in ((256, (8, 8, 4), (3, 5, 7), ((1, 2), (2, 6), (3, 12))),
-                              (512, (8, 8, 2, 2), (3, 7, 11), ((1, 3, 5),) * 3)):           # generators (bf16x3)
-        shapes.add((192, C0, 7, 1, 0))
-        ch = C0
-        for u in ups:
-            shapes.add((ch, ch // 2 * u, 2, 1, 0))                                          # ConvTranspose phase rows
-            ch //= 2
-            for kk, dd in zip(ks, dils):
-                for d in set(dd) | {1}:
-                    shapes.add((ch, ch, kk, d, 0))
-    out = (C.c_int32 * 12)()
-    for ci, rows, k, dil, tf32 in sorted(shapes):
-        check(lib_built.pb200_debug_mma_plan(ci, rows, k, dil, tf32, out))
-        ok, mt, kc, stage_rows, n_tile, n_tiles, acc_cols, tmem_cols, a_slots, w_slots, n_acc, smem = list(out)
-        assert ok == 1, (ci, rows, k, dil, tf32)
-        assert mt in (128, 256) and ci % kc == 0 and kc % (8 if tf32 else 16) == 0
-        assert n_tile * n_tiles == rows and n_tile % 16 == 0 and n_tile <= 256
-        assert stage_rows >= mt + (k - 1) * dil and stage_rows % 8 == 0
-        assert (mt // 128) * n_acc * acc_cols <= tmem_cols <= 512
-        assert 0 < smem <= 227 * 1024 and 1 <= a_slots <= 2 and 2 <= w_slots <= 4
-        assert n_acc == (3 if tf32 else 1)
-    # shapes the tensor-core path must decline (they fall back to the CUDA-core kernel)
-    for bad in ((192, 29, 1, 1, 1), (1, 192, 1, 1, 1), (100, 64, 3, 1, 0)):
-        check(lib_built.pb200_debug_mma_plan(*bad, out))
-        assert out[0] == 0, bad
-
-
 def test_voicegen_is_deterministic(tmp_path):
     a = voicegen.build("tiny", seed=7)
     b = voicegen.build("tiny", seed=7)

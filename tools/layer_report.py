@@ -38,13 +38,9 @@ else:
 n_l = len(runs[0])
 assert all(len(r) == n_l for r in runs)
 pm.B = a.batch
-# model the kernel that is actually running (the defaults since round 2: second-generation kernel, fp16x3, tensor-map TMA;
-# the first-generation kernels are selected by PIPER_B200_V2=0)
-if os.environ.get("PIPER_B200_V2", "2") != "0":
-    pm.V2, pm.F16 = True, os.environ.get("PIPER_B200_V2_PREC", "f16") == "f16"
-    pm.TMA_CYC = 0.0 if os.environ.get("PIPER_B200_V2_TM", "1") != "0" else 20.0
-elif os.environ.get("PIPER_B200_UNI"):
-    pm.TMA_CYC = 20.0
+# model the kernel that is actually running (default fp16x3 with tensor-map TMA)
+pm.F16 = os.environ.get("PIPER_B200_V2_PREC", "f16") == "f16"
+pm.TMA_CYC = 0.0 if os.environ.get("PIPER_B200_V2_TM", "1") != "0" else 20.0
 rows = []
 for i in range(n_l):
     r = dict(runs[0][i])

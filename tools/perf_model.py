@@ -1,25 +1,21 @@
 """Analytical per-layer model of the headline step (medium voice, 32 utterances, T = 259 ids, T' ~ 509 frames) - runs on
-the CPU, no GPU needed.  For every dense convolution it derives, from the same tiling rules the engine uses
-(conv_mma.cu: mma_plan / persist_cfg):
+the CPU, no GPU needed.  For every dense convolution it derives, from the tiling plan of the tensor-core kernel
+(conv_mma2.cu, through tests/sim/libconv2_sim.so) and its stacked-weight scheme (A_hi x [W_hi;W_lo] + A_lo x W_hi, two
+instructions per k-step):
 
   * t_hbm   - layer-wise algorithmic bytes (SURVEY 8d) / measured copy peak
-  * t_mma   - tcgen05.mma issue time: instructions per tile x cost(N), cost fitted to tools/mma_bench.py
-              (48 / 66 / 103 cycles at N = 32 / 128 / 256  ->  (4096 + 32 N) / 128 + 8: the SS-form instruction is paced by
+  * t_mma   - tcgen05.mma issue time: instructions per tile x cost(N) (mma_cost below: the SS-form instruction is paced by
               reading its A (128 x 32 B) and B (N x 32 B) operands from shared memory at 128 B/clk)
   * t_w     - weight units streamed L2 -> shared memory per tile / ~42 B/clk/SM (6300 B/clk chip-wide)
+  * t_tma   - issue time of the activation-row bulk copies by the TMA thread: rows per tile x ~20 cycles with uniform
+              issue (PIPER_B200_V2_TM=0; tools/layer_report.py sets 0 for the tensor-map loads: one copy per channel chunk)
   * wave quantisation: tiles are dealt to 148 persistent CTAs, the slowest CTA sets the time
 
-and prints them next to the measured per-family conv time of the final round-1 bench line.  The gap between
-max(t_hbm, t_mma, t_w) and the measurement is what per-tile latency, the epilogue and the converters cost today.
+and prints them next to the measured per-family conv time of the final round-1 bench line (profiles/bench_r1_final.json,
+the first-generation kernel, kept for reference).
 
-  * t_tma   - issue time of the activation-row bulk copies by the single TMA thread: rows per tile x ~150 cycles in the
-              shipped kernel (address arithmetic in vector registers + R2UR + ELECT loop, DESIGN.md section 8), ~20 cycles
-              with uniform issue (experimental kernels)
-
-usage: python tools/perf_model.py [--stack] [--v2 [--f16]]
-  --stack  model the [W_hi;W_lo] N-stacked two-instruction scheme on the shipped tiling
-  --v2     project the experimental second-generation kernel (conv_mma2.cu): its own plan (tests/sim/libconv2_sim.so),
-           stacked weights, uniform TMA issue; --f16: fp16x3 operands for every family (K = 16 per instruction)
+usage: python tools/perf_model.py [--std]
+  --std    bf16x3 for the generator and tf32x3 elsewhere (PIPER_B200_V2_PREC=std) instead of fp16x3 for every family
 """
 import json, math, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -27,10 +23,8 @@ HBM = 6572.2e9
 CLK = 1.965e9
 SMS = 148
 L2_B_PER_CLK_SM = 6300.0 / SMS
-STACK = "--stack" in sys.argv
-V2 = "--v2" in sys.argv
-F16 = "--f16" in sys.argv
-TMA_CYC = 20.0 if V2 else 150.0   # (tools/layer_report.py sets 0 for the tensor-map kernel: one copy per channel chunk)
+F16 = "--std" not in sys.argv
+TMA_CYC = 20.0                    # (tools/layer_report.py sets 0 for the tensor-map kernel: one copy per channel chunk)
 
 B, T, TP = 32, 259, 509          # utterances, ids, frames per utterance (bench: 4 071 680 samples / 256 / 32 = 497..520)
 
@@ -39,35 +33,15 @@ def mma_cost(n):                  # cycles per tcgen05.mma, M = 128, K = 32 byte
     # round 2, measured with the kernel's exact instruction stream (tools/probe/mma_probe.cu, profiles/r02_mma_probe_*.txt):
     # 64 / 49 / ~40 cycles at N = 128 / 64 / 32 = the larger of the tensor-pipe floor 128 N / 256 and the time its A
     # (128 x 32 B) and B (N x 32 B) operands take to leave shared memory at 128 B/clk.  (Round 1 fitted (4096 + 32 N) / 128 + 8
-    # to tools/mma_bench.py, which included the issue loop.)
+    # to a microbenchmark that included the issue loop.)
     return max(n / 2.0, 32.0 + n / 4.0)
-
-
-def plan(ci, rows, k, dil, tf32):
-    """n_tile, n_tiles, mt as chosen by mma_plan + persist_cfg (conv_mma.cu)."""
-    n_acc = 3 if tf32 else 1
-    max_tile = (128 if (ci * k >= 900 and rows >= 256) else 64) if tf32 else 256
-    nt = 1
-    while rows // nt > max_tile or rows % nt or (rows // nt) % 16:
-        nt += 1
-    n_tile = rows // nt
-    acc_cols = ((n_tile + 31) & ~31) if tf32 else (32 if n_tile <= 32 else 64 if n_tile <= 64 else 128 if n_tile <= 128 else 256)
-    es = 4 if tf32 else 2
-    for slots in (2, 1):
-        for m in (256, 128):
-            if tf32 and m != 128:
-                continue
-            if m // 128 * n_acc * acc_cols * slots > 512:
-                continue
-            return n_tile, nt, m
-    return n_tile, nt, 128
 
 
 _sim = None
 
 
 def plan_v2(ci, rows, k, dil, prec, chains):
-    """(n_tile, n_tiles, mt, kc) from the experimental kernel's own planner."""
+    """(n_tile, n_tiles, mt, kc) from the kernel's own planner."""
     global _sim
     import ctypes as C
     if _sim is None:
@@ -81,20 +55,13 @@ def plan_v2(ci, rows, k, dil, prec, chains):
 
 def layer(name, fam, ci, rows, k, dil, L, tf32, extra_rw=0.0, up=1):
     """L: output positions per utterance *before* the pixel shuffle (ConvT computes L_in positions x rows = co*stride)."""
-    if V2:
-        prec = 2 if F16 else (1 if tf32 else 0)
-        n_tile, n_tiles, mt, kc = plan_v2(ci, rows, k, dil, prec, 2 if tf32 else 1)
-        es = 4 if prec == 1 else 2
-    else:
-        n_tile, n_tiles, mt = plan(ci, rows, k, dil, tf32)
-        es = 4 if tf32 else 2
-    kstep = 32 // es // 2 * 2 if False else (8 if es == 4 else 16)
+    prec = 2 if F16 else (1 if tf32 else 0)
+    n_tile, n_tiles, mt, kc = plan_v2(ci, rows, k, dil, prec, 2 if tf32 else 1)
+    es = 4 if prec == 1 else 2
+    kstep = 8 if es == 4 else 16
     tiles = math.ceil(L / mt) * B * n_tiles
     per_cta = math.ceil(tiles / SMS)
-    if STACK or V2:   # A_hi x [W_hi;W_lo] (N doubled) + A_lo x W_hi
-        per_k = mma_cost(2 * n_tile) + mma_cost(n_tile)
-    else:
-        per_k = 3 * mma_cost(n_tile)
+    per_k = mma_cost(2 * n_tile) + mma_cost(n_tile)   # A_hi x [W_hi;W_lo] (N doubled) + A_lo x W_hi
     mma_tile = (mt // 128) * (ci // kstep) * k * per_k
     w_tile = 2 * ci * k * n_tile * es
     t_mma = per_cta * mma_tile / CLK
@@ -147,12 +114,10 @@ if __name__ == "__main__":
         f["hbm"] += r["t_hbm"]; f["mma"] += r["t_mma"]; f["w"] += r["t_w"]; f["tma"] += r["t_tma"]; f["n"] += 1
         f["bound"] += max(r["t_hbm"], r["t_mma"], r["t_w"])
         f["all"] += max(r["t_hbm"], r["t_mma"], r["t_w"], r["t_tma"])
-    what = ("second-generation kernel, " + ("fp16x3 everywhere" if F16 else "bf16x3 / tf32x3") + ", stacked weights, uniform TMA issue (PROJECTION)") if V2 \
-        else ("N-stacked [W_hi;W_lo] + A_lo x W_hi (2 instructions per k-step)" if STACK else "three instructions per k-step (shipped)")
+    what = "tensor-core kernel, " + ("fp16x3 everywhere" if F16 else "bf16x3 / tf32x3") + ", stacked weights, uniform TMA issue"
     print(f"\nscheme: {what}")
     print(f"{'family':12s} {'launches':>8s} {'sum t_hbm':>10s} {'sum t_mma':>10s} {'sum t_w':>9s} {'sum t_tma':>10s} {'max w/o tma':>12s} {'max with tma':>13s} {'measured':>9s}  ms per step")
     for k, f in fam.items():
         print(f"{k:12s} {f['n']:8d} {f['hbm'] * 1e3:10.3f} {f['mma'] * 1e3:10.3f} {f['w'] * 1e3:9.3f} {f['tma'] * 1e3:10.3f} {f['bound'] * 1e3:12.3f} "
               f"{f['all'] * 1e3:13.3f} {meas.get(k, float('nan')):9.3f}")
-    if V2:
-        print("(measured = the shipped kernel, for reference; the projection has not been measured)")
+    print("(measured = the round-1 kernel, for reference)")

@@ -3,7 +3,8 @@
 Part 1 — which split-precision scheme does each layer family tolerate?  Products are formed exactly (fp64 accumulate)
 from operands rounded like the tensor core sees them: single-pass TF32, bf16x3 (hi*hi + hi*lo + lo*hi), tf32x3.
 Part 2 — the tensor core adds into its fp32 accumulator with truncation (round toward zero): emulate that per k-step
-and evaluate the two mitigations shipped in conv_mma.cu (separate correction accumulator, K split into chains).
+and evaluate the two mitigations against it (separate correction accumulator, K split into chains; conv2_body.inl keeps
+a correction accumulator per K-chain).
 
 Part 3 - FP16 operands: hi = fp16(x), lo = fp16(x - hi) keeps 22 mantissa bits at kind::f16's K = 16 per instruction,
 i.e. tf32x3-class accuracy at bf16x3 cost (conv2_body.inl PREC_F16); with the accumulator truncation emulated as well.
