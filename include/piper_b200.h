@@ -143,6 +143,26 @@ int pb200_debug_conv1d(int32_t backend, const float* x, int32_t B, int32_t ci, i
                        const float* bias, int32_t co, int32_t k, int32_t dil, float pre_slope, const float* resid,
                        float* y);
 
+/* Kernel-level test hook: ONE conv launch with any fused epilogue, on a ragged batch, through back end `backend` (numbered
+ * as above), packed and launched the way the engine launches a layer.  The descriptor (the field order of the CPU model's
+ * conv2_sim_run in tests/sim/conv2_sim.cpp, without its plan fields):
+ *   desc = {ci, rows, k, dil, pad, q_extra, pre (0 none / 1 leaky-relu with `slope`), epi (kernels.cuh Epilogue), split,
+ *           first, up, up_pad, mrf, mrf_n, len_scale, cs_x, cs_y, cs_y2, cs_r, C_y, C_y2, C_r, flags}
+ * x has ci channels, y / y2 / r have C_y / C_y2 / C_r channels; cs_* are the row pitches in floats (multiples of 4).
+ * Item-major layout [B][C][cs], or with PB200_CONV_FLAT the engine's flat layout [C][B][cs] (item b at column b * cs of
+ * every channel row; the tensor-core kernel then tiles the concatenated time axis where the engine would).  Item b is
+ * valid on [0, len[b] * len_scale).  w [rows][ci][k] (a ConvTranspose already lowered to rows = C_out * up stride-phase
+ * rows), bias [rows] or NULL, bias_item [B][bias_item_stride] (per-item rows added to the bias) or NULL.  y, y2 and r are
+ * uploaded whole and y, y2 copied back whole, so a caller can prefill them and see every store; pass NULL for a buffer the
+ * epilogue does not use.  PB200_CONV_Y_IS_R: the launch reads r from y and writes it in place (WN, SUBFROM; r unused).
+ * PB200_CONV_LATENCY: the latency plan of the tensor-core kernel (two K-chains).  A launch the engine never makes
+ * (odd rows for GATE, rows not a multiple of up, a shape the tensor-core plan declines, ...) is an error. */
+#define PB200_CONV_DESC_LEN 23
+enum { PB200_CONV_Y_IS_R = 1, PB200_CONV_FLAT = 2, PB200_CONV_LATENCY = 4 };
+int pb200_debug_conv(int32_t backend, const int32_t desc[PB200_CONV_DESC_LEN], float slope, const float* x, const float* w,
+                     const float* bias, const float* bias_item, int32_t bias_item_stride, const int32_t* len, int32_t B,
+                     float* y, float* y2, const float* r);
+
 /* Host-only (no GPU): tiling and packed weights of the fused MRF stage (csrc/mrf_fused.cu, engine mask bit 16) for
  * upsample stage `stage` of a voice; fuse_post != 0 plans it with conv_post + tanh fused behind it.
  * plan = {ok, n_chains, n_steps, pair, hv, to, k[3], dil[3][6], post_k}; w = bf16 tap tiles in consumption order,

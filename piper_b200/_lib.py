@@ -56,6 +56,9 @@ SYMBOLS = {
     "pb200_debug_conv1d": (C.c_int, [C.c_int32, _p(C.c_float), C.c_int32, C.c_int32, C.c_int32, _p(C.c_float),
                                      _p(C.c_float), C.c_int32, C.c_int32, C.c_int32, C.c_float, _p(C.c_float),
                                      _p(C.c_float)]),
+    "pb200_debug_conv": (C.c_int, [C.c_int32, _p(C.c_int32), C.c_float, _p(C.c_float), _p(C.c_float), _p(C.c_float),
+                                   _p(C.c_float), C.c_int32, _p(C.c_int32), C.c_int32, _p(C.c_float), _p(C.c_float),
+                                   _p(C.c_float)]),
     "pb200_debug_mrf_pack": (C.c_int, [C.c_char_p, C.c_int32, C.c_int32, _p(C.c_int32), _p(C.c_uint8), _p(C.c_int64), _p(C.c_float),
                                        _p(C.c_int64)]),
     "pb200_release": (None, [C.c_void_p, C.c_void_p]),

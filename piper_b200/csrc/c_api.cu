@@ -253,72 +253,184 @@ int pb200_set_mma(pb200_voice* v, int32_t on) {
     if (_e != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(_e)); \
   } while (0)
 
+}  // extern "C"
+
+namespace {
+
+// device allocations of one test-hook call, freed on every exit path
+struct DevArena {
+  std::vector<void*> ptrs;
+  ~DevArena() {
+    for (void* p : ptrs) cudaFree(p);
+  }
+  template <class T>
+  T* upload(const T* host, size_t n) {
+    if (!host || n == 0) return nullptr;
+    void* d = nullptr;
+    CK(cudaMalloc(&d, n * sizeof(T)));
+    ptrs.push_back(d);
+    CK(cudaMemcpy(d, host, n * sizeof(T), cudaMemcpyHostToDevice));
+    return static_cast<T*>(d);
+  }
+};
+
+[[noreturn]] void conv_reject(const std::string& why) { throw std::runtime_error("pb200_debug_conv: " + why); }
+
+// One conv launch on host arrays, packed and launched the way Engine::conv does it (include/piper_b200.h)
+void debug_conv(int backend, const int32_t* d, float slope, const float* x, const float* w, const float* bias,
+                const float* bias_item, int bias_item_stride, const int32_t* len, int B, float* y, float* y2, const float* r) {
+  using namespace pb200;
+  if (backend < 0 || backend > 6) conv_reject("backend " + std::to_string(backend) + " is not 0..6");
+  if (!d || !x || !w || !len || B <= 0) conv_reject("null argument");
+  const int ci = d[0], rows = d[1], k = d[2], dil = d[3], pad = d[4], q_extra = d[5], pre = d[6], epi = d[7];
+  const int split = d[8], first = d[9], up = d[10], up_pad = d[11], mrf = d[12], mrf_n = d[13], len_scale = d[14];
+  const int flags = d[22];
+  const bool alias = flags & PB200_CONV_Y_IS_R, flat = flags & PB200_CONV_FLAT, latency = flags & PB200_CONV_LATENCY;
+  const int cs_x = d[15], cs_y = d[16], cs_y2 = d[17], C_y = d[19], C_y2 = d[20];
+  const int cs_r = alias ? cs_y : d[18], C_r = alias ? C_y : d[21];          // y == r: r is y
+  if (ci <= 0 || rows <= 0 || k <= 0 || dil <= 0 || pad < 0 || q_extra < 0 || len_scale <= 0 || up <= 0)
+    conv_reject("bad shape");
+  if (epi < EPI_BIAS || epi > EPI_MRF) conv_reject("unknown epilogue " + std::to_string(epi));
+  if (pre != PRE_NONE && pre != PRE_LRELU) conv_reject("unknown pre-activation " + std::to_string(pre));
+  // what the engine never launches
+  if (epi == EPI_GATE && rows % 2) conv_reject("GATE needs an even number of rows");
+  if (epi == EPI_UPSAMPLE ? rows % up != 0 : up != 1) conv_reject("rows % up != 0, or up != 1 without UPSAMPLE");
+  if (q_extra && epi != EPI_UPSAMPLE) conv_reject("q_extra without UPSAMPLE");
+  if (epi == EPI_WN && (split < 0 || split > rows || split % 16)) conv_reject("WN split must be a multiple of 16 in [0, rows]");
+  if (epi == EPI_MRF && (mrf < 0 || mrf > 2 || mrf_n <= 0)) conv_reject("bad MRF mode");
+  if (alias && epi != EPI_WN && epi != EPI_SUBFROM) conv_reject("y == r only for WN and SUBFROM");
+  if (bias_item && bias_item_stride < rows) conv_reject("bias_item stride shorter than rows");
+  // which buffers the epilogue reads and writes, and how many channels of each
+  const bool uses_r = epi == EPI_RES || epi == EPI_WN || epi == EPI_SUBFROM || epi == EPI_MRF;
+  const bool uses_y2 = epi == EPI_MRF || (epi == EPI_WN && split < rows);
+  const bool uses_y = epi != EPI_MRF && !(epi == EPI_WN && split == 0);
+  const int need_y = epi == EPI_GATE ? rows / 2 : epi == EPI_UPSAMPLE ? rows / up : epi == EPI_WN ? split : rows;
+  const int need_r = epi == EPI_WN ? split : rows, need_y2 = epi == EPI_WN ? rows - split : rows;
+  if (uses_y && (!y || C_y < need_y)) conv_reject("y needs " + std::to_string(need_y) + " channels");
+  if (uses_y2 && (!y2 || C_y2 < need_y2)) conv_reject("y2 needs " + std::to_string(need_y2) + " channels");
+  if (uses_r && ((!alias && !r) || (alias && !y) || C_r < need_r)) conv_reject("r needs " + std::to_string(need_r) + " channels");
+  int max_in = 0;
+  for (int b = 0; b < B; ++b) {
+    if (len[b] < 0) conv_reject("negative length");
+    max_in = std::max(max_in, len[b] * len_scale);
+  }
+  const int max_len = max_in + q_extra;
+  // pitches: 16-byte rows (the CUDA-core kernel stages x with 16-byte copies); every valid column inside its row
+  for (int cs : {cs_x, cs_y, cs_y2, cs_r})
+    if (cs < 0 || cs % 4) conv_reject("pitches must be non-negative multiples of 4 floats");
+  if (cs_x < max_in) conv_reject("x pitch shorter than the longest item");
+  if (uses_y && cs_y < (epi == EPI_UPSAMPLE ? max_in * up : max_len)) conv_reject("y pitch too short");
+  if (uses_y2 && cs_y2 < max_len) conv_reject("y2 pitch too short");
+  if (uses_r && cs_r < max_len) conv_reject("r pitch too short");
+  // the tensor-core plan, as Engine::conv2_layer makes it: 1, 3 = bf16x3; 2, 4 = tf32x3 (2 chains); 5 = fp16x3 (1 chain);
+  // 6 = fp16x3 (2 chains); the latency plan (conv2_layer variant 1) takes two chains whatever the back end
+  Conv2Layer l;
+  if (backend) {
+    const int prec = (backend == 1 || backend == 3) ? 0 : (backend == 2 || backend == 4) ? 1 : 2;
+    const int chains = latency || backend == 2 || backend == 4 || backend == 6 ? 2 : 1;
+    if (!conv2_plan(ci, rows, k, dil, prec, chains, l)) conv_reject("shape not supported by the tensor-core conv");
+  }
+
+  // weights in the engine's [ci][k][rows_p] layout (voice.cc), then the tensor-core packing of the plan
+  const int rows_p = (rows + 3) & ~3;
+  std::vector<float> pk(size_t(ci) * k * rows_p, 0.f);
+  for (int i = 0; i < ci; ++i)
+    for (int j = 0; j < k; ++j)
+      for (int o = 0; o < rows; ++o) pk[(size_t(i) * k + j) * rows_p + o] = w[(size_t(o) * ci + i) * k + j];
+  std::vector<uint8_t> packed;
+  if (backend) {
+    packed.resize(l.w_bytes);
+    conv2_pack(pk.data(), ci, k, rows_p, l, packed.data());
+  }
+
+  // buffers: item-major [B][C][cs] or flat [C][B][cs] (the engine's flat layout: item b at b * cs of every channel row)
+  DevArena m;
+  const size_t nx = size_t(B) * ci * cs_x, ny = size_t(B) * C_y * cs_y, ny2 = size_t(B) * C_y2 * cs_y2, nr = size_t(B) * C_r * cs_r;
+  float* dx = m.upload(x, nx);
+  float* dy = uses_y || alias ? m.upload(y, ny) : nullptr;
+  float* dy2 = uses_y2 ? m.upload(y2, ny2) : nullptr;
+  float* dr = alias ? dy : uses_r ? m.upload(r, nr) : nullptr;
+  const float* dbias = m.upload(bias, size_t(rows));
+  const float* dbi = bias_item ? m.upload(bias_item, size_t(B - 1) * bias_item_stride + rows) : nullptr;
+  const int* dlen = m.upload(len, size_t(B));
+  auto view = [&](float* p, int C, int cs) {
+    return flat ? View{p, (long long)cs, B * cs} : View{p, (long long)C * cs, cs};
+  };
+  const View vx = view(dx, ci, cs_x), vy = view(dy, C_y, cs_y), vy2 = view(dy2, C_y2, cs_y2),
+             vr = alias ? vy : view(dr, C_r, cs_r);
+
+  if (backend == 0) {
+    ConvArgs a;
+    a.x = vx; a.y = vy; a.y2 = vy2; a.r = vr;
+    a.w = m.upload(pk.data(), pk.size());
+    a.bias = dbias; a.bias_item = dbi; a.bias_item_stride = bias_item_stride;
+    a.len = dlen; a.len_scale = len_scale;
+    a.ci = ci; a.rows = rows; a.rows_p = rows_p; a.k = k; a.dil = dil; a.pad = pad; a.q_extra = q_extra;
+    a.pre = pre; a.slope = slope; a.epi = epi; a.split = split; a.first = first;
+    a.up = up; a.up_pad = up_pad; a.mrf = mrf; a.mrf_n = mrf_n;
+    launch_conv1d(a, B, max_len, nullptr);
+  } else {
+    MmaConvArgs a;
+    a.x = vx; a.y = vy; a.y2 = vy2; a.r = vr;
+    a.w = m.upload(packed.data(), packed.size());
+    a.bias = dbias; a.bias_item = dbi; a.bias_item_stride = bias_item_stride;
+    a.len = dlen; a.len_scale = len_scale;
+    a.ci = ci; a.rows = rows; a.k = k; a.dil = dil; a.pad = pad; a.q_extra = q_extra;
+    a.pre = pre; a.slope = slope; a.epi = epi; a.split = split; a.first = first;
+    a.up = up; a.up_pad = up_pad; a.mrf = mrf; a.mrf_n = mrf_n;
+    // one launch item on the concatenated time axis under the conditions of Engine::conv (engine.cu), per-item tiles otherwise
+    auto same_layout = [&](const View& v) { return v.p == nullptr || (v.bs == vx.bs && v.cs == vx.cs); };
+    const bool flat_launch = flat && len_scale == 1 && q_extra == 0 && vx.bs < (long long)vx.cs && vx.bs >= 2 &&
+                             ((long long)vx.cs + 1024) * vx.bs < (1LL << 32) && same_layout(a.y) && same_layout(a.y2) &&
+                             same_layout(a.r);
+    if (flat_launch) {
+      a.flat_tg = int(vx.bs);
+      a.flat_n = B;
+      launch_conv2(a, l, 1, B * int(vx.bs), nullptr);
+    } else {
+      launch_conv2(a, l, B, max_len, nullptr);
+    }
+  }
+  CK(cudaGetLastError());
+  CK(cudaDeviceSynchronize());
+  if (uses_y || alias) CK(cudaMemcpy(y, dy, ny * 4, cudaMemcpyDeviceToHost));
+  if (uses_y2) CK(cudaMemcpy(y2, dy2, ny2 * 4, cudaMemcpyDeviceToHost));
+}
+
+}  // namespace
+
+extern "C" {
+
+int pb200_debug_conv(int32_t backend, const int32_t desc[PB200_CONV_DESC_LEN], float slope, const float* x, const float* w,
+                     const float* bias, const float* bias_item, int32_t bias_item_stride, const int32_t* len, int32_t B,
+                     float* y, float* y2, const float* r) {
+  return guarded([&] { debug_conv(backend, desc, slope, x, w, bias, bias_item, bias_item_stride, len, B, y, y2, r); });
+}
+
 int pb200_debug_conv1d(int32_t backend, const float* x, int32_t B, int32_t ci, int32_t L, const float* w,
                        const float* bias, int32_t co, int32_t k, int32_t dil, float pre_slope, const float* resid,
                        float* y) {
   return guarded([&] {
     using namespace pb200;
     if (!x || !w || !y || B <= 0 || L <= 0) throw std::runtime_error("pb200_debug_conv1d: bad argument");
-    if (backend < 0 || backend > 6)
-      throw std::runtime_error("pb200_debug_conv1d: backend " + std::to_string(backend) + " is not 0..6");
-    const int Lp = (L + 3) & ~3, pad = dil * (k - 1) / 2, rows_p = (co + 3) & ~3;
-    float *dx = nullptr, *dy = nullptr, *dr = nullptr, *dw = nullptr, *db = nullptr;
-    int* dlen = nullptr;
-    uint8_t* dw16 = nullptr;
-    CK(cudaMalloc(&dx, size_t(B) * ci * Lp * 4));
-    CK(cudaMalloc(&dy, size_t(B) * co * Lp * 4));
-    CK(cudaMemset(dy, 0, size_t(B) * co * Lp * 4));
-    CK(cudaMemcpy2D(dx, size_t(Lp) * 4, x, size_t(L) * 4, size_t(L) * 4, size_t(B) * ci, cudaMemcpyHostToDevice));
+    // every item L long, rows padded to a 16-byte pitch, y zeroed; only the valid columns come back
+    const int Lp = (L + 3) & ~3;
+    std::vector<float> xp(size_t(B) * ci * Lp, 0.f), yp(size_t(B) * co * Lp, 0.f), rp;
+    for (size_t row = 0; row < size_t(B) * ci; ++row) std::memcpy(&xp[row * Lp], x + row * L, size_t(L) * 4);
     if (resid) {
-      CK(cudaMalloc(&dr, size_t(B) * co * Lp * 4));
-      CK(cudaMemcpy2D(dr, size_t(Lp) * 4, resid, size_t(L) * 4, size_t(L) * 4, size_t(B) * co, cudaMemcpyHostToDevice));
+      rp.assign(size_t(B) * co * Lp, 0.f);
+      for (size_t row = 0; row < size_t(B) * co; ++row) std::memcpy(&rp[row * Lp], resid + row * L, size_t(L) * 4);
     }
-    if (bias) {
-      CK(cudaMalloc(&db, size_t(co) * 4));
-      CK(cudaMemcpy(db, bias, size_t(co) * 4, cudaMemcpyHostToDevice));
-    }
-    std::vector<int> lens(B, L);
-    CK(cudaMalloc(&dlen, size_t(B) * 4));
-    CK(cudaMemcpy(dlen, lens.data(), size_t(B) * 4, cudaMemcpyHostToDevice));
-    View vx{dx, (long long)ci * Lp, Lp}, vy{dy, (long long)co * Lp, Lp}, vr{dr, (long long)co * Lp, Lp};
-    if (backend == 0) {
-      std::vector<float> pk(size_t(ci) * k * rows_p, 0.f);
-      for (int i = 0; i < ci; ++i)
-        for (int j = 0; j < k; ++j)
-          for (int o = 0; o < co; ++o) pk[(size_t(i) * k + j) * rows_p + o] = w[(size_t(o) * ci + i) * k + j];
-      CK(cudaMalloc(&dw, pk.size() * 4));
-      CK(cudaMemcpy(dw, pk.data(), pk.size() * 4, cudaMemcpyHostToDevice));
-      ConvArgs a;
-      a.x = vx; a.y = vy; a.r = vr; a.w = dw; a.bias = db; a.len = dlen; a.len_scale = 1;
-      a.ci = ci; a.rows = co; a.rows_p = rows_p; a.k = k; a.dil = dil; a.pad = pad;
-      a.pre = pre_slope != 0.f ? PRE_LRELU : PRE_NONE; a.slope = pre_slope;
-      a.epi = resid ? EPI_RES : EPI_BIAS;
-      launch_conv1d(a, B, L, nullptr);
-    } else {
-      // tensor-core kernel (conv_mma2.cu): 1, 3 = bf16x3; 2, 4 = tf32x3 (2 chains); 5 = fp16x3 (1 chain); 6 = fp16x3 (2 chains)
-      const int prec = (backend == 1 || backend == 3) ? 0 : (backend == 2 || backend == 4) ? 1 : 2;
-      const int chains = (backend == 2 || backend == 4 || backend == 6) ? 2 : 1;
-      Conv2Layer l;
-      if (!conv2_plan(ci, co, k, dil, prec, chains, l))
-        throw std::runtime_error("shape not supported by the tensor-core conv");
-      std::vector<float> pk(size_t(ci) * k * rows_p, 0.f);
-      for (int i = 0; i < ci; ++i)
-        for (int j = 0; j < k; ++j)
-          for (int o = 0; o < co; ++o) pk[(size_t(i) * k + j) * rows_p + o] = w[(size_t(o) * ci + i) * k + j];
-      std::vector<uint8_t> packed(l.w_bytes);
-      conv2_pack(pk.data(), ci, k, rows_p, l, packed.data());
-      CK(cudaMalloc(&dw16, packed.size()));
-      CK(cudaMemcpy(dw16, packed.data(), packed.size(), cudaMemcpyHostToDevice));
-      MmaConvArgs a;
-      a.x = vx; a.y = vy; a.r = vr; a.w = dw16; a.bias = db; a.len = dlen; a.len_scale = 1;
-      a.ci = ci; a.rows = co; a.k = k; a.dil = dil; a.pad = pad;
-      a.pre = pre_slope != 0.f ? PRE_LRELU : PRE_NONE; a.slope = pre_slope;
-      a.epi = resid ? EPI_RES : EPI_BIAS;
-      launch_conv2(a, l, B, L, nullptr);
-    }
-    CK(cudaDeviceSynchronize());
-    CK(cudaMemcpy2D(y, size_t(L) * 4, dy, size_t(Lp) * 4, size_t(L) * 4, size_t(B) * co, cudaMemcpyDeviceToHost));
-    cudaFree(dx); cudaFree(dy); cudaFree(dr); cudaFree(dw); cudaFree(db); cudaFree(dlen); cudaFree(dw16);
+    const std::vector<int32_t> lens(B, L);
+    int32_t d[PB200_CONV_DESC_LEN] = {};
+    d[0] = ci; d[1] = co; d[2] = k; d[3] = dil; d[4] = dil * (k - 1) / 2;
+    d[6] = pre_slope != 0.f ? PRE_LRELU : PRE_NONE;
+    d[7] = resid ? EPI_RES : EPI_BIAS;
+    d[10] = 1; d[13] = 1; d[14] = 1;
+    d[15] = Lp; d[16] = Lp; d[18] = resid ? Lp : 0; d[19] = co; d[21] = resid ? co : 0;
+    debug_conv(backend, d, pre_slope, xp.data(), w, bias, nullptr, 0, lens.data(), B, yp.data(), nullptr,
+               resid ? rp.data() : nullptr);
+    for (size_t row = 0; row < size_t(B) * co; ++row) std::memcpy(y + row * L, &yp[row * Lp], size_t(L) * 4);
   });
 }
 

@@ -257,5 +257,39 @@ def debug_conv1d(backend: int, x, w, bias=None, dil: int = 1, pre_slope: float =
     return y
 
 
+EPILOGUES = dict(BIAS=0, RELU=1, RES=2, GATE=3, WN=4, SUBFROM=5, UPSAMPLE=6, MRF=7)   # csrc/kernels.cuh Epilogue
+
+
+def debug_conv(backend: int, x, w, lens, *, epi: str = "BIAS", bias=None, bias_item=None, dil: int = 1, pad=None,
+               slope=None, y=None, y2=None, r=None, y_is_r: bool = False, split: int = 0, first: int = 0, up: int = 1,
+               up_pad: int = 0, q_extra: int = 0, mrf: int = 0, mrf_n: int = 1, len_scale: int = 1, flat: bool = False,
+               latency: bool = False):
+    """One conv launch with a fused epilogue on a ragged batch, packed and launched as the engine does it (unit-test hook,
+    pb200_debug_conv in include/piper_b200.h).  x, y, y2, r are [B][C][pitch], or [C][B][pitch] with flat=True; item b is
+    valid on [0, lens[b] * len_scale).  w [rows][ci][k]; bias [rows]; bias_item [B][stride]; slope: leaky-relu before the
+    conv (None: no pre-activation); pad defaults to dil * (k - 1) // 2.  y and y2 are in/out: the launch starts from copies
+    of them, which come back whole as (y, y2) (None for a buffer not passed).  y_is_r: r is read from y, in place."""
+    def f32(a):
+        return None if a is None else np.ascontiguousarray(a, np.float32)
+    x, w, r, bias, bias_item = f32(x), f32(w), f32(r), f32(bias), f32(bias_item)
+    y = None if y is None else np.array(y, np.float32, order="C")
+    y2 = None if y2 is None else np.array(y2, np.float32, order="C")
+    lens = np.ascontiguousarray(lens, np.int32)
+    rows, ci, k = w.shape
+    ch = 0 if flat else 1                                  # index of the channel axis
+
+    def dims(a):
+        return (0, 0) if a is None else (a.shape[ch], a.shape[2])
+    (_, cs_x), (C_y, cs_y), (C_y2, cs_y2), (C_r, cs_r) = dims(x), dims(y), dims(y2), dims(r)
+    assert x.shape[ch] == ci and x.shape[1 - ch] == len(lens)
+    desc = (C.c_int32 * 23)(ci, rows, k, dil, dil * (k - 1) // 2 if pad is None else pad, q_extra, 0 if slope is None else 1,
+                            EPILOGUES[epi], split, first, up, up_pad, mrf, mrf_n, len_scale, cs_x, cs_y, cs_y2, cs_r,
+                            C_y, C_y2, C_r, (1 if y_is_r else 0) | (2 if flat else 0) | (4 if latency else 0))
+    check(_lib.load().pb200_debug_conv(backend, desc, 0.0 if slope is None else slope, _fptr(x), _fptr(w), _fptr(bias),
+                                       _fptr(bias_item), 0 if bias_item is None else bias_item.shape[1],
+                                       lens.ctypes.data_as(C.POINTER(C.c_int32)), len(lens), _fptr(y), _fptr(y2), _fptr(r)))
+    return y, y2
+
+
 def launch_count() -> int:
     return int(_lib.load().pb200_launch_count())
